@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the many-chain WALNUTS hot path: gradient evals/sec and min-ESS/sec.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1], the config the metric is quoted on): 1000-d ill-conditioned diagonal
 Gaussian, sigma = logspace(-2, 2, 1000), 65 536 chains PER GPU (weak scaling), WALNUTSpy driver with
@@ -20,6 +20,9 @@ ONE JSON line (rank 0):
                    C3 funnel, C4 logistic regression, C5 Stock-Watson (131 072 chains per GPU = 1 048 576 on 8 GPUs)
                    and 1 048 576 C2 chains on one GPU -- each with value, e2e, roofline, cpu_baseline, clocks
   strong_scaling   the headline workload with 65 536 chains in TOTAL split over the N GPUs (N > 1)
+`--dump-outputs DIR` writes what the headline's last timed step handed back (float64 .npy files, see
+headline_outputs) so that two builds can be compared output for output; the inputs depend only on the arguments.
+With N > 1 GPUs the dump holds rank 0's chains only.
 `--impl reference` times the CPU restatement of the reference's Python implementation (oracle/walnutspy_oracle.py;
 the reference itself is Python and cannot travel to the GPU box) on all host cores.
 """
@@ -35,6 +38,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+if __name__ in ("__main__", "__mp_main__"):      # the script and its CPU-arm workers
+    sys.dont_write_bytecode = True    # the bench writes nothing into the tree it runs from (which may be read-only)
 
 SEED = 20251017
 D = 1000
@@ -75,6 +80,9 @@ CONFIG_ORDER = ["c1", "c2_nuts", "c3", "c4", "c5", "c2_1m"]
 # coordinate (sigma = 100) has an autocorrelation time of ~700 transitions at this tuning, so the chains must be long;
 # the estimator pools 592 x N_GPU chains that start from exact draws of the target.
 ESS_CHAINS, ESS_DRAWS = 592, 2048
+# --dump-outputs: draws of up to 65 536 chains and positions of up to 4 096 (one position is 8 KB at d = 1000);
+# larger batches are sampled with a fixed seed.  At most 8.4 + 32.8 MB.
+DUMP_DRAW_CHAINS, DUMP_STATE_CHAINS = 65536, 4096
 
 
 def sigma_vec():
@@ -206,7 +214,7 @@ def _cpu_worker(args):
         kind = {"fixed": wo.FIXED, "D": wo.ADAPT_D, "R2P": wo.ADAPT_R2P}[spec["integrator"]]
         ref_name = {"fixed": "fixedLeapFrog", "D": "adaptLeapFrogD", "R2P": "adaptLeapFrogR2P"}[spec["integrator"]]
         if impl == "reference":
-            from oracle import ref_loader        # the REAL WALNUTS.py / adaptiveIntegrators.py (oracle/_ref or /root/reference)
+            from oracle import ref_loader        # the REAL WALNUTS.py / adaptiveIntegrators.py ($WALNUTS_REFERENCE or oracle/_ref)
         it = 1
         while True:
             t0 = time.perf_counter()
@@ -363,9 +371,25 @@ def _traffic(name, chains, iters):
         return {"traffic": None}
 
 
-def gpu_leg(env, name, steps, warmup, chains=None, e2e=True, fp64_peak=None, keep_draws=False):
+def headline_outputs(env, cb, draws, grad_evals):
+    """What a caller of the device-resident path receives from one step: the monitored draws (iters, chains, monitor),
+    the chain positions (chains, d) and the gradient evaluations (forward, backward) of the step.  Chains beyond
+    DUMP_DRAW_CHAINS / DUMP_STATE_CHAINS are sampled (seed SEED, sorted rows), so the sample depends only on the
+    chain count."""
+    n = cb.n_chains
+
+    def rows(k):
+        return np.arange(n) if n <= k else np.sort(np.random.default_rng(SEED).choice(n, k, replace=False))
+    state = env.torch.empty((n, cb.d), dtype=env.torch.float64, device=env.dev)
+    cb.get_state(state)
+    return {"draws": draws[:, env.torch.as_tensor(rows(DUMP_DRAW_CHAINS), device=env.dev)].cpu().numpy(),
+            "positions": state[env.torch.as_tensor(rows(DUMP_STATE_CHAINS), device=env.dev)].cpu().numpy(),
+            "grad_evals": np.array(grad_evals, dtype=np.float64)}
+
+
+def gpu_leg(env, name, steps, warmup, chains=None, e2e=True, fp64_peak=None, dump=False):
     """Device-resident timing (+ e2e through pinned host buffers) of one workload; returns the reduced dict on
-    every rank."""
+    every rank.  dump=True: out["_outputs"] = headline_outputs() of the last timed step."""
     from walnuts_b200.sampler import pinned_empty
     torch = env.torch
     spec = WORKLOADS[name]
@@ -397,6 +421,7 @@ def gpu_leg(env, name, steps, warmup, chains=None, e2e=True, fp64_peak=None, kee
     clocks = sampler.stop() if sampler else None
     launches = steps * cb.last_launches()
     dev_ms = float(sum(kernel_ms))
+    outputs = headline_outputs(env, cb, draws, (f, b)) if dump else None
 
     # ---- e2e: the same steps through HOST buffers, copies inside the timed region; the chains are split over two
     # handles so that the copies of one half overlap the kernel of the other -------------------------------------
@@ -473,8 +498,8 @@ def gpu_leg(env, name, steps, warmup, chains=None, e2e=True, fp64_peak=None, kee
     if e2e_wall_max > 0:
         out["e2e"] = {"value": e2e_evals_all / e2e_wall_max, "unit": "grad_evals/s", "h2d_bytes_per_step": h2d,
                       "d2h_bytes_per_step": d2h, "handles_per_gpu": len(halves)}
-    if keep_draws:
-        out["_draws"] = draws
+    if dump:
+        out["_outputs"] = outputs
     return out
 
 
@@ -550,7 +575,9 @@ def reference_arm(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=8)
+    ap.add_argument("--steps", type=int, default=8,
+                    help="timed steps of the headline workload (exactly); the config legs cap it at their steps_cap, "
+                         "strong scaling at 5, and the reference arm takes it as a maximum -- each reports its own count")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--chains", type=int, default=CHAINS_PER_GPU, help="headline chains per GPU")
@@ -561,7 +588,11 @@ def main():
     ap.add_argument("--ess-draws", type=int, default=ESS_DRAWS)
     ap.add_argument("--ref-budget", type=float, default=60.0, help="seconds per core of the reference arm")
     ap.add_argument("--ref-min-transitions", type=int, default=4, help="timed transitions per core of the reference arm")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline's outputs of its last timed step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl ours and --steps >= 1")
 
     if args.impl == "reference":
         if int(os.environ.get("RANK", "0")) == 0:
@@ -576,7 +607,11 @@ def main():
     except Exception:
         peak, peak_src = 148 * 64 * 2 * 1.965e9 / 1e12, "nominal 148 SM x 64 FMA/clk x 1.965 GHz (fallback)"
 
-    head = gpu_leg(env, "c2", args.steps, args.warmup, chains=args.chains, fp64_peak=peak)
+    head = gpu_leg(env, "c2", args.steps, args.warmup, chains=args.chains, fp64_peak=peak, dump=bool(args.dump_outputs))
+    if args.dump_outputs and env.rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for key, arr in head.pop("_outputs").items():
+            np.save(os.path.join(args.dump_outputs, key + ".npy"), arr)
     names = CONFIG_ORDER if args.configs == "all" else ([] if args.configs == "none" else args.configs.split(","))
     configs = {}
     for name in names:

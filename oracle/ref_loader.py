@@ -1,7 +1,7 @@
-"""Load the REAL reference (when /root/reference is present) and run it under an injected RNG.
+"""Load the REAL reference (a checkout named by $WALNUTS_REFERENCE, or the copy staged in oracle/_ref) and run it
+under an injected RNG.
 
-TEST / BASELINE INFRASTRUCTURE ONLY; used by tests/golden/make_golden.py to generate the committed fixtures, by
-tests/test_oracle_golden.py to pin the restatements in oracle/ against the live reference, and by
+TEST / BASELINE INFRASTRUCTURE ONLY; used by tests/golden/make_golden.py to generate the committed fixtures and by
 `bench.py --impl reference` (the CPU arm) through the copy staged in oracle/_ref by oracle/stage_ref.py.  The product
 (walnuts_b200/) never imports it.
 
@@ -20,14 +20,9 @@ import numpy as np
 from . import philox
 
 def _ref_root():
-    """$WALNUTS_REFERENCE, else /root/reference (the build container), else the copy staged by oracle/stage_ref.py
-    (oracle/_ref: the only form in which the reference reaches the GPU box)."""
-    env = os.environ.get("WALNUTS_REFERENCE")
-    if env:
-        return env
-    if os.path.isfile("/root/reference/WALNUTSpy/WALNUTS.py"):
-        return "/root/reference"
-    return os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
+    """$WALNUTS_REFERENCE (a checkout of bob-carpenter/walnuts), else the copy staged by oracle/stage_ref.py
+    (oracle/_ref)."""
+    return os.environ.get("WALNUTS_REFERENCE") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 
 REF_ROOT = _ref_root()

@@ -10,9 +10,8 @@ adaptLeapFrogR2P) in the streaming form the CUDA kernels use:
     both ends of every finished subtree; only the left ends are ever read, :575-587);
   * running min/max replace the 2**M arrays Hs/Ifs/Ibs/cs/lwts (WALNUTS.py:170-174).
 
-Pinned against the reference itself: tests/test_oracle_golden.py (live when /root/reference is present, else the committed goldens of tests/golden/make_golden.py) runs the real
-WALNUTS.py (when /root/reference is present) under the same RNG and requires bit-identical
-samples and diagnostics; tests/golden/*.npz hold reference outputs for boxes without it.
+Pinned against the reference itself: tests/test_oracle_golden.py requires bit-identical samples and diagnostics
+against tests/golden/*.npz, outputs of the real WALNUTS.py under the same RNG (tests/golden/make_golden.py).
 
 All reference quirks of SURVEY.md row A14 are reproduced (cited inline).
 """

@@ -1,8 +1,7 @@
-"""Generate the golden fixtures by running the REAL reference (/root/reference) under the Philox RNG
-shims of oracle/ref_loader.py and oracle/package_oracle.py.  Run from the repo root in the build
-container (the GPU box has no /root/reference):
+"""Generate the golden fixtures by running the REAL reference (a bob-carpenter/walnuts checkout) under the Philox RNG
+shims of oracle/ref_loader.py and oracle/package_oracle.py.  Run from the repo root:
 
-    PYTHONPATH=. python tests/golden/make_golden.py
+    WALNUTS_REFERENCE=<checkout> PYTHONPATH=. python tests/golden/make_golden.py
 
 Each .npz stores the inputs (config, q0, seed, chain) and the reference's own outputs.
 """
