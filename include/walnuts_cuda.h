@@ -70,6 +70,14 @@ extern "C" {
 
 #define WN_DIAG_COLS 24 /* WALNUTS.py:180,670-693 */
 
+/* kernel families (wn_last_plan): each is a separate set of template instantiations, picked per call */
+#define WN_FAMILY_WPY 0   /* plain WALNUTSpy transition, adaptLeapFrogD / adaptLeapFrogR2P              */
+#define WN_FAMILY_PKG 1   /* package mode (walnuts/walnuts.py)                                          */
+#define WN_FAMILY_ADAPT 2 /* every integrator behind the runtime kind: adaptYoshidaD, warm-up adaptation,
+                             orbit statistics                                                          */
+#define WN_FAMILY_EXT 3   /* adaptLeapFrogFlowD / adaptImplicitMidpointD / adaptRescaledLeapFrogD        */
+#define WN_FAMILY_NUTS 4  /* plain WALNUTSpy transition, fixedLeapFrog (plain NUTS)                     */
+
 typedef struct wn_handle wn_handle;
 
 typedef struct wn_config {
@@ -174,6 +182,10 @@ int wn_free_pinned(void* p);
 int wn_last_kernel_ms(wn_handle* h, float* ms);
 int wn_last_launches(wn_handle* h, int64_t* n);
 int wn_last_grad_evals(wn_handle* h, uint64_t* forward, uint64_t* backward);
+
+/* The launch plan of the last wn_run* call: out = {WN_FAMILY_*, threads per chain G, coordinate pairs per thread E2,
+ * threads per block NT}.  A handle that has not run yet reports {-1, 0, 0, 0}.  For testing and tuning. */
+int wn_last_plan(wn_handle* h, int32_t out[4]);
 
 /* Cross-chain moments of the current state over this handle's chains: mean[d], var[d]
  * (unbiased).  Multi-GPU callers reduce (n, sum, sumsq) themselves. */

@@ -51,6 +51,8 @@ def oracle_target(name, d, data=None):
         return otargets.funnel10
     if name == "corr_gauss":
         return otargets.corr_gauss
+    if name == "funnel_pkg":       # the package-mode funnel density under the WALNUTSpy lpFun protocol
+        return lambda q, hessian=False: [otargets.funnel_lpdf(q), otargets.funnel_grad(q)]
     if name == "logreg":
         return otargets.make_logreg(data["X"], data["y"], float(np.asarray(data.get("tau", 1.0)).ravel()[0]))
     if name == "dense_gauss":

@@ -35,7 +35,8 @@ def test_corr_gauss(cuda_lib, integrator):
 
 @pytest.mark.parametrize("integrator", EXT)
 def test_diag_gauss_block_per_chain(cuda_lib, integrator):
-    """d = 1000 ill-conditioned Gaussian (BASELINE config 2 shape): one 256-thread CTA per chain."""
+    """d = 1000 ill-conditioned Gaussian (BASELINE config 2 shape): the ext plan there is 64 threads per chain with 8
+    coordinate pairs each, one chain per 64-thread CTA (64 x 8, NT = 64)."""
     d = 1000
     sigma = np.logspace(-2, 2, d)
     data = {"inv_var": 1.0 / sigma ** 2}

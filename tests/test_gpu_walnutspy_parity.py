@@ -14,7 +14,8 @@ EXACT_COLS = [0, 1, 4, 5, 6, 7, 8, 9, 12, 13, 19, 20, 21, 22]
 FLOAT_COLS = [2, 3, 10, 11, 14, 15, 16, 17, 18, 23]
 
 
-def run_cuda(name, q0, integrator, H0, delta, M, n_iter, seed, minC=0, maxC=10, data=None):
+def run_cuda(name, q0, integrator, H0, delta, M, n_iter, seed, minC=0, maxC=10, data=None, plan=None):
+    """`plan`: the (family, G, E2, NT) the call must run on (ChainBatch.last_plan), or None."""
     from walnuts_b200 import ChainBatch
     n_chains, d = q0.shape
     with ChainBatch(name, d, n_chains, integrator=integrator, H0=H0, delta=delta, M=M, minC=minC, maxC=maxC,
@@ -22,12 +23,14 @@ def run_cuda(name, q0, integrator, H0, delta, M, n_iter, seed, minC=0, maxC=10, 
         cb.set_state(q0)
         out = cb.run(n_iter, draws=True, diag=True)
         state = cb.get_state()
+        if plan is not None:
+            assert cb.last_plan() == tuple(plan), f"ran on plan {cb.last_plan()}, expected {tuple(plan)}"
     return out, state
 
 
 def check(name, q0, integrator, H0, delta, M, n_iter, seed=1234, chains=None, minC=0, maxC=10, data=None,
-          float_rtol=1e-9):
-    out, state = run_cuda(name, q0, integrator, H0, delta, M, n_iter, seed, minC, maxC, data)
+          float_rtol=1e-9, plan=None):
+    out, state = run_cuda(name, q0, integrator, H0, delta, M, n_iter, seed, minC, maxC, data, plan)
     chains = list(range(q0.shape[0])) if chains is None else chains
     draws_o, diag_o = oracle_walnutspy(name, q0, integrator, H0, delta, M, n_iter, seed, chains, minC, maxC, data)
     # diagonal Gaussians: every coordinate against ITS standard deviation (north_star: 1e-10 relative)
@@ -47,7 +50,7 @@ def check(name, q0, integrator, H0, delta, M, n_iter, seed=1234, chains=None, mi
     return diag_o
 
 
-def check_forced(name, q0, integrator, H0, delta, M, n_iter, seed=1234, minC=0, maxC=10, data=None):
+def check_forced(name, q0, integrator, H0, delta, M, n_iter, seed=1234, minC=0, maxC=10, data=None, plan=None):
     """Teacher-forced parity for chaotic targets: every transition starts from the ORACLE's previous
     state, so each of the n_iter transitions is compared on identical inputs (rounding differences of
     one implementation cannot be amplified across transitions by the dynamics)."""
@@ -62,6 +65,8 @@ def check_forced(name, q0, integrator, H0, delta, M, n_iter, seed=1234, minC=0, 
         for it in range(n_iter):
             cb.set_state(prev)
             out = cb.run(1, draws=True, diag=True)
+            if plan is not None:
+                assert cb.last_plan() == tuple(plan), f"ran on plan {cb.last_plan()}, expected {tuple(plan)}"
             ok, err = close(out["draws"][0], draws_o[it])
             worst = max(worst, err)
             assert ok, f"transition {it}: draws differ, max rel err {err:.3e}"

@@ -9,12 +9,13 @@ TARGETS = {"std_normal": 0, "diag_gauss": 1, "funnel": 2, "logreg": 3, "stock_wa
 MODE_WALNUTSPY, MODE_PACKAGE = 0, 1
 INT_FIXED, INT_D, INT_R2P = 0, 1, 2
 DIAG_COLS = 24
+FAMILIES = {"wpy": 0, "pkg": 1, "adapt": 2, "ext": 3, "nuts": 4}      # WN_FAMILY_* (wn_last_plan)
 ERRORS = {-1: "WN_EINVAL", -2: "WN_ECUDA", -3: "WN_ENOMEM", -4: "WN_EUNSUPPORTED", -5: "WN_ESTATE"}
 
 # every symbol include/walnuts_cuda.h declares
 SYMBOLS = ["wn_abi_version", "wn_target_id", "wn_register_user_target", "wn_create", "wn_destroy", "wn_set_data", "wn_set_aux", "wn_set_adapt", "wn_set_state",
            "wn_get_state", "wn_run", "wn_run_stats", "wn_run_async", "wn_sync", "wn_run_host_async", "wn_alloc_pinned", "wn_free_pinned", "wn_last_kernel_ms", "wn_last_launches",
-           "wn_last_grad_evals", "wn_moments", "wn_stream", "wn_last_error", "wn_fp64_peak",
+           "wn_last_plan", "wn_last_grad_evals", "wn_moments", "wn_stream", "wn_last_error", "wn_fp64_peak",
            "wn_comm_load", "wn_comm_unique_id", "wn_comm_init_rank", "wn_comm_init_all", "wn_comm_destroy",
            "wn_ess_rhat", "wn_moments_all"]
 
@@ -71,6 +72,7 @@ def load():
     lib.wn_free_pinned.argtypes = [vp]
     lib.wn_last_kernel_ms.argtypes = [vp, P(C.c_float)]
     lib.wn_last_launches.argtypes = [vp, P(C.c_int64)]
+    lib.wn_last_plan.argtypes = [vp, P(C.c_int32)]
     lib.wn_last_grad_evals.argtypes = [vp, P(C.c_uint64), P(C.c_uint64)]
     lib.wn_moments.argtypes = [vp, dp, dp]
     lib.wn_comm_load.argtypes = [C.c_char_p]

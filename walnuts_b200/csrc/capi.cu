@@ -47,20 +47,24 @@ static int user_family(const wn_config& c) { return c.mode == WN_MODE_PACKAGE ? 
 
 // `general`: the call needs the kernels that carry every integrator behind the runtime kind plus the adaptation and
 // orbit-statistics code ("adapt" family): warm-up iterations, wn_run_stats with orbit buffers, adaptYoshidaD.
-static bool pick_plan(const wn_config& c, bool general, LaunchPlan& p) {
+// `fam` receives the family (FAM_*) the plan was picked from.
+static bool pick_plan(const wn_config& c, bool general, LaunchPlan& p, int& fam) {
   if (c.target >= WN_TARGET_USER_BASE) {
     const UserTarget* u = user_target(c.target);
     if (!u || u->d != c.d) return false;
     int pkg = 0;
     p.fn = nullptr;   // launched inside the plug-in
-    u->plan(user_family(c), &p.G, &p.E2, &p.NT, &p.smem, &pkg);
+    fam = user_family(c);
+    u->plan(fam, &p.G, &p.E2, &p.NT, &p.smem, &pkg);
     p.package = pkg != 0;
     return true;
   }
-  if (c.mode == WN_MODE_PACKAGE) return wn_pick_plan_pkg(c, p);
-  if (c.integrator > WN_INT_YOSHIDA) return wn_pick_plan_ext(c, p);
-  if (general || c.integrator == WN_INT_YOSHIDA) return wn_pick_plan_adapt(c, p);
-  return c.integrator == WN_INT_FIXED ? wn_pick_plan_nuts(c, p) : wn_pick_plan_wpy(c, p);
+  if (c.mode == WN_MODE_PACKAGE) { fam = FAM_PKG; return wn_pick_plan_pkg(c, p); }
+  if (c.integrator > WN_INT_YOSHIDA) { fam = FAM_EXT; return wn_pick_plan_ext(c, p); }
+  if (general || c.integrator == WN_INT_YOSHIDA) { fam = FAM_ADAPT; return wn_pick_plan_adapt(c, p); }
+  if (c.integrator == WN_INT_FIXED) { fam = FAM_NUTS; return wn_pick_plan_nuts(c, p); }
+  fam = FAM_WPY;
+  return wn_pick_plan_wpy(c, p);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -171,7 +175,8 @@ int wn_create(const wn_config* cfg, wn_handle** out) {
   h->iter_done = c.first_iteration > 1 ? (uint32_t)c.first_iteration - 1u : 0u;
   h->iter_base = h->iter_done;
   LaunchPlan p;
-  if (!pick_plan(c, false, p)) return fail(h, WN_EUNSUPPORTED, "no CUDA kernel for this target/dimension");
+  int fam;
+  if (!pick_plan(c, false, p, fam)) return fail(h, WN_EUNSUPPORTED, "no CUDA kernel for this target/dimension");
   CUDA_TRY(h, cudaSetDevice(c.device));
   cudaDeviceProp prop;
   CUDA_TRY(h, cudaGetDeviceProperties(&prop, c.device));
@@ -376,8 +381,9 @@ static int run_async_impl(wn_handle* h, int64_t n_iter, double* d_draws, double*
     return fail(h, WN_ESTATE, "dense_gauss needs data key precision [d*d]");
   if (c.mode == WN_MODE_PACKAGE && !h->d_inv_mass) return fail(h, WN_ESTATE, "package mode needs data key inv_mass");
   LaunchPlan p;
+  int fam;
   const bool adapting = h->d_adapt_state != nullptr && h->iter_done < (uint32_t)h->warmup_iter;
-  if (!pick_plan(c, adapting || d_omin != nullptr, p)) return fail(h, WN_EUNSUPPORTED, "no CUDA kernel for this target/dimension");
+  if (!pick_plan(c, adapting || d_omin != nullptr, p, fam)) return fail(h, WN_EUNSUPPORTED, "no CUDA kernel for this target/dimension");
   CUDA_TRY(h, cudaSetDevice(c.device));
   const UserTarget* ut = user_target(c.target);
   int occ = 0;
@@ -479,6 +485,7 @@ static int run_async_impl(wn_handle* h, int64_t n_iter, double* d_draws, double*
   if (h->d_cost) h->have_cost = true;
   h->iter_done += (uint32_t)n_iter;
   h->last_launches = 1;
+  h->last_plan[0] = fam; h->last_plan[1] = p.G; h->last_plan[2] = p.E2; h->last_plan[3] = p.NT;
   return WN_OK;
 }
 
@@ -573,6 +580,11 @@ int wn_last_kernel_ms(wn_handle* h, float* ms) {
 int wn_last_launches(wn_handle* h, int64_t* n) {
   if (!h || !n) return WN_EINVAL;
   *n = h->last_launches;
+  return WN_OK;
+}
+int wn_last_plan(wn_handle* h, int32_t out[4]) {
+  if (!h || !out) return WN_EINVAL;
+  memcpy(out, h->last_plan, sizeof(h->last_plan));
   return WN_OK;
 }
 int wn_last_grad_evals(wn_handle* h, uint64_t* forward, uint64_t* backward) {

@@ -20,7 +20,8 @@ struct LaunchPlan {
   bool package;
 };
 
-enum { FAM_WPY = 0, FAM_PKG = 1, FAM_ADAPT = 2, FAM_EXT = 3, FAM_NUTS = 4 };
+enum { FAM_WPY = WN_FAMILY_WPY, FAM_PKG = WN_FAMILY_PKG, FAM_ADAPT = WN_FAMILY_ADAPT, FAM_EXT = WN_FAMILY_EXT,
+       FAM_NUTS = WN_FAMILY_NUTS };
 
 template <int G, int E2>
 using StdNormalT = DiagGaussT<G, E2, true>;

@@ -218,6 +218,13 @@ class ChainBatch:
         self._check(self._lib.wn_last_launches(self._h, C.byref(n)), "wn_last_launches")
         return int(n.value)
 
+    def last_plan(self):
+        """(family, G, E2, NT) of the last run: the kernel family (_ffi.FAMILIES), threads per chain, coordinate pairs
+        per thread and threads per block; family -1 before the first run."""
+        out = (C.c_int32 * 4)()
+        self._check(self._lib.wn_last_plan(self._h, out), "wn_last_plan")
+        return tuple(int(x) for x in out)
+
     def last_grad_evals(self):
         f, b = C.c_uint64(), C.c_uint64()
         self._check(self._lib.wn_last_grad_evals(self._h, C.byref(f), C.byref(b)), "wn_last_grad_evals")
