@@ -22,5 +22,5 @@ for r in range(a.reps):
     cb.run_device(a.iters)
     f, b = cb.last_grad_evals(); ms = cb.last_kernel_ms()
     res.append((f + b) / (ms * 1e-3))
-print("WN_VARIANT=%s chains=%d %s: %.4g grad evals/s (%.2f TFLOP/s algorithmic), last %.1f ms" % (
-    os.environ.get("WN_VARIANT", "-"), a.chains, a.integrator, max(res), max(res) * 12e3 / 1e12, ms))
+print("chains=%d %s: %.4g grad evals/s (%.2f TFLOP/s algorithmic), last %.1f ms" % (
+    a.chains, a.integrator, max(res), max(res) * 12e3 / 1e12, ms))

@@ -4,7 +4,6 @@
 
 #include <cmath>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <deque>
 #include <mutex>
@@ -449,7 +448,6 @@ static int run_async_impl(wn_handle* h, int64_t n_iter, double* d_draws, double*
     P.p2prob = 1.0 - h->adHtarget; P.adTarget = h->adTarget; P.adQuant = h->adQuant;
     P.adapt_state = h->d_adapt_state; P.adapt_hist = h->d_adapt_hist;
     P.maxFPiter = h->maxFPiter; P.FPtol = h->FPtol; P.gradThresh = h->gradThresh;
-    { const char* tv = getenv("WN_TUNE"); P.tune = tv ? atoi(tv) : 0; }
     // once adaptation has run, the adapted per-chain H / delta are the step sizes (WALNUTS.py:137,144)
     P.Hstep = h->d_H; P.delta = h->d_delta; P.state = h->d_state; P.draws = d_draws; P.diag = d_diag;
     P.orbit_min = d_omin; P.orbit_max = d_omax;

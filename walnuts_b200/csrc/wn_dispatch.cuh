@@ -5,8 +5,6 @@
 // "nuts" = fixedLeapFrog only, "wpy" = adaptLeapFrogD / adaptLeapFrogR2P only; adaptYoshidaD, the warm-up adaptation and
 // the orbit statistics run on the "adapt" family (every integrator behind the runtime kind).
 #pragma once
-#include <cstdlib>
-
 #include "../../include/walnuts_cuda.h"
 #include "wn_package.cuh"
 #include "wn_walnutspy.cuh"
@@ -29,19 +27,19 @@ template <int G, int E2>
 using DiagT = DiagGaussT<G, E2, false>;
 
 template <template <int, int> class T, int G, int E2, int NT, int MINB = 1, bool ADAPT = false, bool EXT = false,
-          int KSET = KSET_ANY, bool CTLSM = false, int NSMV = 0>
+          int KSET = KSET_ANY, bool CTLSM = false>
 static LaunchPlan plan_wpy() {
   LaunchPlan p;
-  p.fn = (const void*)walnutspy_kernel<T, G, E2, NT, MINB, ADAPT, EXT, KSET, CTLSM, NSMV>;
+  p.fn = (const void*)walnutspy_kernel<T, G, E2, NT, MINB, ADAPT, EXT, KSET, CTLSM>;
   p.G = G; p.E2 = E2; p.NT = NT;
-  p.smem = (size_t)wpy_smem_doubles<T, G, E2, NT, ADAPT, KSET, NSMV>() * sizeof(double);
+  p.smem = (size_t)wpy_smem_doubles<T, G, E2, NT, ADAPT, KSET>() * sizeof(double);
   p.package = false;
   return p;
 }
 // plain family: the kernel set follows from the family (FAM_NUTS: fixedLeapFrog, FAM_WPY: D / R2P)
-template <int FAM, template <int, int> class T, int G, int E2, int NT, int MINB = 1, bool CTLSM = false, int NSMV = 0>
+template <int FAM, template <int, int> class T, int G, int E2, int NT, int MINB = 1, bool CTLSM = false>
 static LaunchPlan plan_plain() {
-  return plan_wpy<T, G, E2, NT, MINB, false, false, (FAM == FAM_NUTS) ? KSET_FIXED : KSET_ADAPT, CTLSM, NSMV>();
+  return plan_wpy<T, G, E2, NT, MINB, false, false, (FAM == FAM_NUTS) ? KSET_FIXED : KSET_ADAPT, CTLSM>();
 }
 template <template <int, int> class T, int G, int E2, int NT>
 static LaunchPlan plan_pkg() {
@@ -85,10 +83,14 @@ static bool pick_generic(int d, LaunchPlan& p) {
   WN_PICK(512, 4, 512)     // d <= 4096: one 16-warp CTA per chain, one CTA per SM
   return false;
 }
-template <int FAM, template <int, int> class T>
-static bool pick_warp(int d, LaunchPlan& p) {  // targets that need the chain inside one warp
-  if constexpr (FAM == FAM_NUTS || FAM == FAM_PKG) { WN_PICK(1, 6, 128) }
-  else { WN_PICK(8, 1, 128) }
+// targets that need the chain inside one warp; FIRST = false leaves out the first row for a caller that serves those d
+// with a plan of its own
+template <int FAM, template <int, int> class T, bool FIRST = true>
+static bool pick_warp(int d, LaunchPlan& p) {
+  if constexpr (FIRST) {
+    if constexpr (FAM == FAM_NUTS || FAM == FAM_PKG) { WN_PICK(1, 6, 128) }
+    else { WN_PICK(8, 1, 128) }
+  }
   WN_PICK(16, 1, 128)
   WN_PICK(32, 2, 128)
   WN_PICK(32, 8, 128)
@@ -103,21 +105,14 @@ static bool pick_plan_family(const wn_config& c, LaunchPlan& p) {
     case WN_TARGET_DIAG_GAUSS: {
       if constexpr (FAM == FAM_WPY || FAM == FAM_NUTS) {
         if (c.d > 512 && c.d <= 1024) {
-          // BASELINE config 2 (d = 1000); WN_VARIANT selects alternatives kept for comparison (measured in DESIGN.md
-          // section 6; tuning only)
-          const char* v = getenv("WN_VARIANT");
-          switch (v ? atoi(v) : 0) {
-            case 1: p = plan_plain<FAM, DiagT, 64, 8, 64, 1>(); return true;      // 2 warps per chain
-            case 2: p = plan_plain<FAM, DiagT, 128, 4, 128, 3>(); return true;    // 4 warps per chain, 3 blocks / SM
-            default:
-              // D / R2P: 128 threads x 8 coordinates, 4 blocks / SM at 126 registers.  Plain NUTS (level loop): ONE
-              // warp per chain, 32 coordinates per lane, inverse variances in shared memory, gradient recomputed
-              // (DiagSmT) -- no replicated scalar work, no block barrier per leaf pair: 4.8e8 grad evals/s against
-              // 3.5e8 for 4 warps per chain (WN_VARIANT=2) and 1.68e8 for the flat loop of round 1
-              if constexpr (FAM == FAM_NUTS) p = plan_plain<FAM, DiagSmT, 32, 16, 64, 4>();
-              else p = plan_plain<FAM, DiagT, 128, 4, 128, 4>();
-              return true;
-          }
+          // BASELINE config 2 (d = 1000; the shapes measured against each other are in DESIGN.md section 6).
+          // D / R2P: 128 threads x 8 coordinates, 4 blocks / SM at 126 registers.  Plain NUTS (level loop): ONE warp
+          // per chain, 32 coordinates per lane, inverse variances in shared memory, gradient recomputed (DiagSmT) --
+          // no replicated scalar work, no block barrier per leaf pair: 4.8e8 grad evals/s against 3.5e8 for 4 warps
+          // per chain and 1.68e8 for the flat loop of round 1
+          if constexpr (FAM == FAM_NUTS) p = plan_plain<FAM, DiagSmT, 32, 16, 64, 4>();
+          else p = plan_plain<FAM, DiagT, 128, 4, 128, 4>();
+          return true;
         }
       }
       return pick_generic<FAM, DiagT>(c.d, p);
@@ -130,36 +125,28 @@ static bool pick_plan_family(const wn_config& c, LaunchPlan& p) {
           // different handlers of the state machine most of the time, so a warp issues nearly every instruction for ONE
           // of its chains (measured 1.4 chains per issued instruction with 8 chains per warp): fewer chains per warp
           // with shorter per-thread code win.  Measured at 262 144 chains x 10 transitions, R2P / fixedLeapFrog, ms per
-          // call: 1 thread per chain (WN_VARIANT=1) ~330 / --, 4 threads x 4 coordinates (WN_VARIANT=4, the round-2
-          // default until then) 253 / 99, 8 x 2 (default) 204 / 74, 16 x 2 204 / 79, 32 x 2 243 / 87
-          const char* v = getenv("WN_VARIANT");
-          const int var = v ? atoi(v) : 0;
-          if (var == 1 && c.d <= 12) p = plan_plain<FAM, FunnelT, 1, 6, 128, 1>();
-          else if (var == 5) p = plan_plain<FAM, FunnelT, 4, 2, 128, 1>();
-          else if (var == 4) p = plan_plain<FAM, FunnelT, 4, 2, 128, 4, true>();
-          else p = plan_plain<FAM, FunnelT, 8, 1, 128, 5, true>();
+          // call: 1 thread per chain ~330 / --, 4 threads x 4 coordinates (the round-2 default until then) 253 / 99,
+          // 8 x 2 (shipped) 204 / 74, 16 x 2 204 / 79, 32 x 2 243 / 87
+          p = plan_plain<FAM, FunnelT, 8, 1, 128, 5, true>();
           return true;
         }
+        return pick_warp<FAM, FunnelT, false>(c.d, p);
+      } else {
+        return pick_warp<FAM, FunnelT>(c.d, p);
       }
-      return pick_warp<FAM, FunnelT>(c.d, p);
     case WN_TARGET_FUNNEL_PKG: return pick_warp<FAM, FunnelPkgT>(c.d, p);
     case WN_TARGET_LOGREG: {
       if (c.d > 128) return false;
-      // block-cooperative gradient (8 chains per CTA share every load of X) for the plain WALNUTSpy kernel;
-      // the per-warp version serves package mode / warm-up adaptation / the other integrators and
-      // WN_VARIANT=1 (comparison)
+      // plain WALNUTSpy kernel: FP64 tensor-core gradient with TMA-staged row tiles up to d = 104, the
+      // block-cooperative FMA gradient (8 chains per CTA share every load of X) above; the per-warp version serves
+      // package mode / warm-up adaptation / the other integrators
       if constexpr (FAM == FAM_WPY || FAM == FAM_NUTS) {
-        const char* v = getenv("WN_VARIANT");
-        const int var = v ? atoi(v) : 0;
-        if (var != 1) {
-          // default: FP64 tensor-core gradient with TMA-staged row tiles; WN_VARIANT=2: the FMA-pipe version
-          if (var == 2 || c.d > 104) p = plan_plain<FAM, LogRegCoopT, 32, 2, 256>();
-          else if (c.d <= 32) p = plan_plain<FAM, LogRegMma32T, 32, 2, 256>();
-          else p = plan_plain<FAM, LogRegMma104T, 32, 2, 256>();
-          return true;
-        }
+        if (c.d <= 32) p = plan_plain<FAM, LogRegMma32T, 32, 2, 256>();
+        else if (c.d <= 104) p = plan_plain<FAM, LogRegMma104T, 32, 2, 256>();
+        else p = plan_plain<FAM, LogRegCoopT, 32, 2, 256>();
+      } else {
+        p = plan_for<FAM, LogRegT, 32, 2, 256>();
       }
-      p = plan_for<FAM, LogRegT, 32, 2, 256>();
       return true;
     }
     case WN_TARGET_STOCK_WATSON: {
@@ -169,13 +156,9 @@ static bool pick_plan_family(const wn_config& c, LaunchPlan& p) {
       if (T <= 64 * 4) {
         // 6 blocks / SM (168 registers, 12 warps) measured 9 % faster than 4 blocks at 255 registers
         // (8 blocks / SM at 128 registers: spills, same throughput); round 2: see below
-        if constexpr (FAM == FAM_WPY || FAM == FAM_NUTS) {
-          const char* v = getenv("WN_VARIANT");
-          // measured (C5 shape, R2P): launch bounds for 5 blocks / SM 2.65e8, for 6 blocks / SM 2.53e8 grad evals/s
-          // (4 warps per chain with 2 time steps per thread, 128 / 96 registers: the same 2.63e8)
-          if (v && atoi(v) == 1) p = plan_plain<FAM, StockWatsonT, 64, 7, 64, 6>();
-          else p = plan_plain<FAM, StockWatsonT, 64, 7, 64, 5>();
-        }
+        // measured (C5 shape, R2P): launch bounds for 5 blocks / SM 2.65e8, for 6 blocks / SM 2.53e8 grad evals/s
+        // (4 warps per chain with 2 time steps per thread, 128 / 96 registers: the same 2.63e8)
+        if constexpr (FAM == FAM_WPY || FAM == FAM_NUTS) p = plan_plain<FAM, StockWatsonT, 64, 7, 64, 5>();
         else p = plan_for<FAM, StockWatsonT, 64, 7, 64>();
         return true;
       }
@@ -188,8 +171,7 @@ static bool pick_plan_family(const wn_config& c, LaunchPlan& p) {
       // TMA-staged rows of P; everything else (package mode, warm-up adaptation, other integrators, d > 104) on the
       // per-warp FMA version
       if constexpr (FAM == FAM_WPY || FAM == FAM_NUTS) {
-        const char* v = getenv("WN_VARIANT");
-        if (!(v && atoi(v) == 1) && c.d <= 104) {
+        if (c.d <= 104) {
           if (c.d <= 32) p = plan_plain<FAM, DenseGaussMma32T, 32, 2, 256>();
           else p = plan_plain<FAM, DenseGaussMma104T, 32, 2, 256>();
           return true;

@@ -22,10 +22,8 @@
 //
 // The queue is a scheduling hint only: every chain appears in it exactly once, its random numbers are keyed by (seed,
 // chain id, iteration) and its state is its own, so the draws are bit-identical with and without it
-// (tests/test_gpu_stats.py).  WN_SCHED=0 in the environment turns it off, WN_SCHED=1 keeps step 2 only (A/B
-// measurement).  The sort (cub radix sort of n_chains 32-bit keys) and the two small kernels run on the handle's stream
-// inside the timed region of the call (~40 us at 262 144 chains).
-#include <cstdlib>
+// (tests/test_gpu_stats.py).  The sort (cub radix sort of n_chains 32-bit keys) and the two small kernels run on the
+// handle's stream inside the timed region of the call (~40 us at 262 144 chains).
 #include <cub/cub.cuh>
 
 #include "wn_handle.hpp"
@@ -82,11 +80,10 @@ int wn_sched_prepare(wn_handle* h, int nslot, int chains_per_warp, const unsigne
   *order = nullptr;
   const int n = h->cfg.n_chains;
   const int W = chains_per_warp < 1 ? 1 : chains_per_warp;
-  static const int mode = [] { const char* v = getenv("WN_SCHED"); return v ? atoi(v) : 2; }();
   // every chain has its own slot from the start: the order cannot matter; and a call of a few milliseconds is not
   // worth the sort (the previous call's duration is known after wn_sync)
-  if (mode == 0 || n <= nslot || (h->last_ms > 0.f && h->last_ms < 5.f)) return WN_OK;
-  const int kmax = (mode >= 2 && W > 1) ? (nslot / W) / 16 : 0;
+  if (n <= nslot || (h->last_ms > 0.f && h->last_ms < 5.f)) return WN_OK;
+  const int kmax = (W > 1) ? (nslot / W) / 16 : 0;
   if (!h->d_cost) {
     CUDA_TRY(h, cudaMalloc(&h->d_cost, (size_t)n * sizeof(unsigned int)));
     CUDA_TRY(h, cudaMalloc(&h->d_cost_sorted, (size_t)n * sizeof(unsigned int)));

@@ -73,12 +73,8 @@ struct UserWarpT {
 };
 
 constexpr int WN_USER_E2 = (WN_USER_D + 1) / 2;
-#ifdef WN_USER_FORCE_WARP          // measurement: the warp layout at any d (scripts/user_layout_sweep.py)
-constexpr bool WN_USER_WARP = true;
-#else
 constexpr bool WN_USER_WARP = WN_USER_D > 64;
-#endif
-constexpr int WN_USER_WE2 = (WN_USER_D <= 64) ? 1 : (WN_USER_D <= 256) ? 4 : 8;     // 32 lanes x 2 / 8 / 16 coordinates
+constexpr int WN_USER_WE2 = (WN_USER_D <= 256) ? 4 : 8;     // 32 lanes x 8 / 16 coordinates
 
 // (a template, so that only the layout in use is instantiated)
 template <bool WARP>

@@ -55,8 +55,6 @@ struct RunParams {
   // integratorAuxPar fields of the extended integrators (adaptiveIntegrators.py:36-44); EXT kernels only
   int maxFPiter;
   double FPtol, gradThresh;
-  int tune;              // tuning switches (environment WN_TUNE, read at launch; none in use: an L1 prefetch of the
-                         // deeper left ends under the leapfrog steps measured 3 % slower)
 };
 #define WN_ADAPT_STRIDE 16
 
@@ -106,9 +104,9 @@ enum { KSET_ANY = 0, KSET_FIXED = 1, KSET_ADAPT = 2 };
 // left-end stack levels of the plain-NUTS level loop that live in shared memory (levels 1..NSM; deeper ones in L2 scratch)
 template <int G, int E2, int NT>
 struct NutsCfg {
-  // one level costs 2 * 2 E2 * NT doubles per block: 16 KB for the d = 1000 shape with 128 threads x 8 coordinates;
-  // measured there: 3 levels 3.53e8, 2 levels 3.45e8, 4 levels 3.15e8 grad evals/s (the L1 carve-out shrinks)
-  static constexpr int NSM = (G == 128 && E2 == 4) ? 3 : 2;
+  // one level costs 2 * 2 E2 * NT doubles per block; more levels shrink the L1 carve-out (measured for 4 warps per
+  // chain at d = 1000: 2 levels 3.45e8, 4 levels 3.15e8 grad evals/s)
+  static constexpr int NSM = 2;
 };
 // one warp holds a whole d = 1000 chain (32 coordinates per lane): a level costs 16 KB per chain, one level fits
 template <int NT>
@@ -132,18 +130,18 @@ struct NutsFast {
 };
 // dynamic shared memory of walnutspy_kernel in doubles: checkpoint (or the plain-NUTS left-end slots + uniform buffer),
 // reduction scratch, target
-template <template <int, int> class TargetTT, int G, int E2, int NT, bool ADAPT, int KSET, int NSMV = 0>
+template <template <int, int> class TargetTT, int G, int E2, int NT, bool ADAPT, int KSET>
 __host__ __device__ constexpr int wpy_smem_doubles() {
   using Target = TargetTT<G, E2>;
   constexpr bool NF = NutsFast<Target, G, ADAPT, KSET>::value;
-  return (NF ? 2 * (NSMV ? NSMV : NutsCfg<G, E2, NT>::NSM) : 3) * 2 * E2 * NT + (NF ? 2 * NT : 0) +
+  return (NF ? 2 * NutsCfg<G, E2, NT>::NSM : 3) * 2 * E2 * NT + (NF ? 2 * NT : 0) +
          2 * ((G + 31) / 32) * 8 + Target::smem_doubles(NT);
 }
 
 // CTLSM: the cold control block of chains that SHARE a warp (G < 32) lives in shared memory (one copy per chain)
 // instead of per-thread registers / local memory -- fewer registers, more resident warps (G >= 32 always does).
 template <template <int, int> class TargetTT, int G, int E2, int NT, int MINB = 1, bool ADAPT = false, bool EXT = false,
-          int KSET = KSET_ANY, bool CTLSM = false, int NSMV = 0>
+          int KSET = KSET_ANY, bool CTLSM = false>
 __global__ void __launch_bounds__(NT, MINB) walnutspy_kernel(const __grid_constant__ RunParams P) {
   static_assert(!EXT || ADAPT, "EXT kernels are built with the adaptation code (inactive without wn_set_adapt)");
   static_assert(KSET == KSET_ANY || (!ADAPT && !EXT), "specialised kernel sets exist for the plain family only");
@@ -153,7 +151,7 @@ __global__ void __launch_bounds__(NT, MINB) walnutspy_kernel(const __grid_consta
   using Grp = Group<G>;
   using Target = TargetTT<G, E2>;
   constexpr bool NUTS_FAST = NutsFast<Target, G, ADAPT, KSET>::value;
-  constexpr int NSM = NSMV ? NSMV : NutsCfg<G, E2, NT>::NSM;   // NSMV: tuning override of the shared-memory levels
+  constexpr int NSM = NutsCfg<G, E2, NT>::NSM;
   constexpr bool LAZY = Target::LAZY_ENERGY && KSET != KSET_FIXED;   // plain NUTS consumes every step's energy
   constexpr bool REGRAD = NUTS_FAST && has_regrad<Target>::value;      // g is recomputed, never carried
   // integrator predicates: compile-time where the kernel set fixes them

@@ -97,8 +97,7 @@ def cuda_target(source, d, data=None, name="user", verbose=False):
         raise ValueError("cuda_target: 1 <= d <= 512 (d <= 64: one thread per chain holds the whole vector; "
                          "64 < d <= 512: one warp per chain, the density evaluated by every lane on the whole vector)")
     csrc = os.path.join(_build.HERE, "csrc")
-    force = "#define WN_USER_FORCE_WARP 1\n" if os.environ.get("WN_USER_LAYOUT") == "warp" else ""
-    tu = (f"#define WN_USER_D {d}\n{force}#include \"wn_user_api.cuh\"\n#line 1 \"{name}\"\n{source}\n"
+    tu = (f"#define WN_USER_D {d}\n#include \"wn_user_api.cuh\"\n#line 1 \"{name}\"\n{source}\n"
           "#include \"wn_user_plugin.cuh\"\n")
     h = hashlib.sha256()
     h.update(tu.encode())
