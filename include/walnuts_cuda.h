@@ -184,8 +184,13 @@ int wn_last_launches(wn_handle* h, int64_t* n);
 int wn_last_grad_evals(wn_handle* h, uint64_t* forward, uint64_t* backward);
 
 /* The launch plan of the last wn_run* call: out = {WN_FAMILY_*, threads per chain G, coordinate pairs per thread E2,
- * threads per block NT}.  A handle that has not run yet reports {-1, 0, 0, 0}.  For testing and tuning. */
+ * threads per block NT}.  G > NT means one chain per thread-block cluster of G / NT blocks (std_normal and diag_gauss
+ * above d = 4096).  A handle that has not run yet reports {-1, 0, 0, 0}.  For testing and tuning. */
 int wn_last_plan(wn_handle* h, int32_t out[4]);
+
+/* Chain slots of the last wn_run* launch: the chain groups resident at once (blocks x groups per block, or clusters
+ * when G > NT), at most n_chains.  For testing and tuning. */
+int wn_last_slots(wn_handle* h, int64_t* n);
 
 /* Cross-chain moments of the current state over this handle's chains: mean[d], var[d]
  * (unbiased).  Multi-GPU callers reduce (n, sum, sumsq) themselves. */

@@ -15,7 +15,7 @@ ERRORS = {-1: "WN_EINVAL", -2: "WN_ECUDA", -3: "WN_ENOMEM", -4: "WN_EUNSUPPORTED
 # every symbol include/walnuts_cuda.h declares
 SYMBOLS = ["wn_abi_version", "wn_target_id", "wn_register_user_target", "wn_create", "wn_destroy", "wn_set_data", "wn_set_aux", "wn_set_adapt", "wn_set_state",
            "wn_get_state", "wn_run", "wn_run_stats", "wn_run_async", "wn_sync", "wn_run_host_async", "wn_alloc_pinned", "wn_free_pinned", "wn_last_kernel_ms", "wn_last_launches",
-           "wn_last_plan", "wn_last_grad_evals", "wn_moments", "wn_stream", "wn_last_error", "wn_fp64_peak",
+           "wn_last_plan", "wn_last_slots", "wn_last_grad_evals", "wn_moments", "wn_stream", "wn_last_error", "wn_fp64_peak",
            "wn_comm_load", "wn_comm_unique_id", "wn_comm_init_rank", "wn_comm_init_all", "wn_comm_destroy",
            "wn_ess_rhat", "wn_moments_all"]
 
@@ -73,6 +73,7 @@ def load():
     lib.wn_last_kernel_ms.argtypes = [vp, P(C.c_float)]
     lib.wn_last_launches.argtypes = [vp, P(C.c_int64)]
     lib.wn_last_plan.argtypes = [vp, P(C.c_int32)]
+    lib.wn_last_slots.argtypes = [vp, P(C.c_int64)]
     lib.wn_last_grad_evals.argtypes = [vp, P(C.c_uint64), P(C.c_uint64)]
     lib.wn_moments.argtypes = [vp, dp, dp]
     lib.wn_comm_load.argtypes = [C.c_char_p]

@@ -394,11 +394,37 @@ static int run_async_impl(wn_handle* h, int64_t n_iter, double* d_draws, double*
     CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, p.fn, p.NT, p.smem));
   }
   if (occ < 1) return fail(h, WN_ECUDA, "kernel does not fit on an SM");
-  const int gpb = p.NT / p.G;
-  long long blocks = (long long)h->num_sms * occ;
-  const long long need = ((long long)c.n_chains + gpb - 1) / gpb;
-  if (blocks > need) blocks = need;
-  const int nslot = (int)blocks * gpb;
+  // G > NT: one chain per cluster of CL = G / NT blocks (wn_walnutspy.cuh); a slot is a cluster, and the resident
+  // cluster count comes from the runtime (how many clusters of CL blocks the GPCs hold), not from SMs x blocks per SM
+  const int cl = (p.G > p.NT) ? p.G / p.NT : 1;
+  cudaLaunchAttribute cattr[1];
+  cattr[0].id = cudaLaunchAttributeClusterDimension;
+  cattr[0].val.clusterDim.x = (unsigned)cl;
+  cattr[0].val.clusterDim.y = 1;
+  cattr[0].val.clusterDim.z = 1;
+  cudaLaunchConfig_t lcfg = {};
+  lcfg.blockDim = dim3(p.NT);
+  lcfg.dynamicSmemBytes = p.smem;
+  lcfg.stream = h->stream;
+  lcfg.attrs = cattr;
+  lcfg.numAttrs = 1;
+  long long blocks;
+  int nslot;
+  if (cl > 1) {
+    lcfg.gridDim = dim3((unsigned)cl);
+    int ncl = 0;
+    CUDA_TRY(h, cudaOccupancyMaxActiveClusters(&ncl, p.fn, &lcfg));
+    if (ncl < 1) return fail(h, WN_ECUDA, "no cluster of this kernel fits on the GPU");
+    const long long clusters = (ncl < c.n_chains) ? ncl : c.n_chains;
+    blocks = clusters * cl;
+    nslot = (int)clusters;
+  } else {
+    const int gpb = p.NT / p.G;
+    blocks = (long long)h->num_sms * occ;
+    const long long need = ((long long)c.n_chains + gpb - 1) / gpb;
+    if (blocks > need) blocks = need;
+    nslot = (int)blocks * gpb;
+  }
   const int nvec = p.package ? package_scratch_vectors(c.M) : scratch_vectors(c.M);
   const size_t sbytes = (size_t)nvec * p.E2 * nslot * p.G * sizeof(double2);
   if (sbytes > h->scratch_bytes) {
@@ -457,6 +483,9 @@ static int run_async_impl(wn_handle* h, int64_t n_iter, double* d_draws, double*
     if (ut) {
       const int rc = ut->launch(user_family(c), c.device, &P, (unsigned)blocks, h->stream);
       if (rc) return fail(h, WN_ECUDA, "user target plug-in: kernel launch failed (" + std::to_string(rc) + ")");
+    } else if (cl > 1) {
+      lcfg.gridDim = dim3((unsigned)blocks);
+      CUDA_TRY(h, cudaLaunchKernelExC(&lcfg, p.fn, args));
     } else {
       CUDA_TRY(h, cudaLaunchKernel(p.fn, dim3((unsigned)blocks), dim3(p.NT), args, p.smem, h->stream));
     }
@@ -484,6 +513,7 @@ static int run_async_impl(wn_handle* h, int64_t n_iter, double* d_draws, double*
   h->iter_done += (uint32_t)n_iter;
   h->last_launches = 1;
   h->last_plan[0] = fam; h->last_plan[1] = p.G; h->last_plan[2] = p.E2; h->last_plan[3] = p.NT;
+  h->last_slots = nslot;
   return WN_OK;
 }
 
@@ -583,6 +613,11 @@ int wn_last_launches(wn_handle* h, int64_t* n) {
 int wn_last_plan(wn_handle* h, int32_t out[4]) {
   if (!h || !out) return WN_EINVAL;
   memcpy(out, h->last_plan, sizeof(h->last_plan));
+  return WN_OK;
+}
+int wn_last_slots(wn_handle* h, int64_t* n) {
+  if (!h || !n) return WN_EINVAL;
+  *n = h->last_slots;
   return WN_OK;
 }
 int wn_last_grad_evals(wn_handle* h, uint64_t* forward, uint64_t* backward) {

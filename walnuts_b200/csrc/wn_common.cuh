@@ -1,6 +1,7 @@
 // Common device helpers: Philox4x32-10 streams, chain-group reductions, scratch addressing.
 //
-// Layout idea (DESIGN.md section 3): a chain is owned by a group of G threads (G = 1 .. 256).
+// Layout idea (DESIGN.md section 3): a chain is owned by a group of G threads (G = 1 .. 512 in one CTA, 1024 .. 4096 on
+// a thread-block cluster).
 // Thread t of the group holds E = 2*E2 coordinates in registers: the pairs p = e2*G + t,
 // i.e. coordinates 2p and 2p+1.  All per-chain control state is replicated in the registers of
 // the G threads and is bit-identical across them (reductions return identical values to every
@@ -73,19 +74,89 @@ __device__ __forceinline__ void rng_normal_pair(const RngKey& k, uint32_t stream
 }
 
 // --------------------------------------------------------------------------------------
-// Group reductions.  Every thread of the group receives bit-identical results.
+// Thread-block clusters: barrier and distributed shared memory (DSMEM) reads.
 // --------------------------------------------------------------------------------------
-template <int G>
+// Every thread of every CTA of the cluster arrives (release: its earlier shared AND global writes become visible at
+// cluster scope) and waits for all of them (acquire).  Not `.aligned`: correctness does not rest on warp convergence.
+// SASS (sm_100a, CUDA 12.9): MEMBAR.ALL.GPU + UCGABAR_ARV, then UCGABAR_WAIT + CCTL.IVALL (the release fences at GPU
+// scope, the acquire invalidates L1), and ld.shared::cluster below becomes a generic LD.E.64 -- the same as the
+// cooperative_groups form (this_cluster().sync(), map_shared_rank), so the explicit PTX saves neither.
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release;\n\tbarrier.cluster.wait.acquire;" ::: "memory");
+}
+__device__ __forceinline__ uint32_t cluster_rank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+__device__ __forceinline__ uint32_t dsmem_addr(const void* p, uint32_t rank) {
+  uint32_t a;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(a) : "r"((uint32_t)__cvta_generic_to_shared(p)), "r"(rank));
+  return a;
+}
+__device__ __forceinline__ double ld_dsmem(const double* p, uint32_t rank) {
+  double v;
+  asm volatile("ld.shared::cluster.f64 %0, [%1];" : "=d"(v) : "r"(dsmem_addr(p, rank)) : "memory");
+  return v;
+}
+__device__ __forceinline__ uint32_t ld_dsmem(const uint32_t* p, uint32_t rank) {
+  uint32_t v;
+  asm volatile("ld.shared::cluster.u32 %0, [%1];" : "=r"(v) : "r"(dsmem_addr(p, rank)) : "memory");
+  return v;
+}
+
+// --------------------------------------------------------------------------------------
+// Group reductions.  Every thread of the group receives bit-identical results.
+// NTB: threads of the group in ONE CTA.  G > NTB: the group spans a cluster of CL = G / NTB CTAs (one chain per
+// cluster); each reduction first reduces within the CTA exactly as a one-CTA group does, then folds the CL partials
+// through DSMEM in rank order, so every thread of every CTA computes the same sum in the same order.
+// --------------------------------------------------------------------------------------
+template <int G, int NTB = G>
 struct Group {
+  static constexpr int CL = (G > NTB) ? G / NTB : 1;
   static constexpr int LANES = (G < 32) ? G : 32;
-  static constexpr int WARPS = (G + 31) / 32;
+  static constexpr int WARPS = (((CL > 1) ? NTB : G) + 31) / 32;   // warps of the group in one CTA
+  // shared reduction scratch: two halves of WARPS * 8 doubles, and for a cluster group two halves of 8 doubles that
+  // the other CTAs read (the CTA's published partials)
+  static constexpr int RED_DOUBLES = 2 * WARPS * 8 + ((CL > 1) ? 2 * 8 : 0);
+
+  // Cluster stage (CL > 1): x holds the CTA's NV partials, identical in every thread of the CTA.  Thread 0 publishes
+  // them in half `parity` of the CTA's exchange, one cluster barrier, then every thread folds the CL CTAs' partials in
+  // rank order.  The caller flips `parity` afterwards.
+  // Reuse of a half: reduction n + 2 rewrites the half that reduction n published.  Its writer (thread 0) has passed
+  // the cluster barrier of reduction n + 1 by then, and no thread arrives there before it has finished its DSMEM
+  // reads of reduction n -- so every read of a half precedes its next write.  (Further cluster barriers in between,
+  // e.g. a broadcast or a vote, only add order.)
+  template <int NV, class Op>
+  __device__ __forceinline__ static void cluster_fold(double (&x)[NV], double* red, int parity, Op op) {
+    double* xb = red + 2 * WARPS * 8 + parity * 8;
+    if (threadIdx.x == 0) {
+#pragma unroll
+      for (int k = 0; k < NV; ++k) xb[k] = x[k];
+    }
+    cluster_sync();
+#pragma unroll
+    for (int k = 0; k < NV; ++k) {
+      double s = ld_dsmem(xb + k, 0u);
+#pragma unroll
+      for (int r = 1; r < CL; ++r) s = op(s, ld_dsmem(xb + k, (uint32_t)r));
+      x[k] = s;
+    }
+  }
+  struct Plus {
+    __device__ __forceinline__ double operator()(double a, double b) const { return a + b; }
+  };
+  struct MaxN {
+    __device__ __forceinline__ double operator()(double a, double b) const { return maxn2(a, b); }
+  };
 
   __device__ __forceinline__ static unsigned mask() {
     if constexpr (G >= 32) return 0xffffffffu;
     else return ((1u << G) - 1u) << ((threadIdx.x & 31u) & ~(unsigned)(G - 1));
   }
 
-  // red: shared scratch of 2 * WARPS * 8 doubles (G > 32 only: one chain per block), two halves used alternately
+  // red: shared scratch of RED_DOUBLES doubles (G > 32 only: one chain per block, or per cluster when CL > 1 -- then
+  // each CTA holds its own scratch, with the cluster exchange after the two CTA halves), two halves used alternately
   // (`parity`).  EVERY reduction, whatever its number of values, takes the half at red + parity * WARPS * 8: with a
   // value-count-dependent offset the half of one reduction overlapped the other half of the previous one, and a warp
   // that had passed the barrier could overwrite partial sums a slower warp was still reading (racecheck, round 2).
@@ -115,6 +186,7 @@ struct Group {
           for (int ww = 1; ww < WARPS; ++ww) s += buf[ww * NV + k];
           x[k] = s;
         }
+        if constexpr (CL > 1) cluster_fold<NV>(x, red, parity, Plus());
         parity ^= 1;
       }
     }
@@ -148,6 +220,7 @@ struct Group {
         for (int ww = 1; ww < WARPS; ++ww) s += buf[ww * 4 + i];
         x[i] = s;
       }
+      if constexpr (CL > 1) cluster_fold<4>(x, red, parity, Plus());
       parity ^= 1;
     } else {
       x[0] = __shfl_sync(0xffffffffu, k, 0);
@@ -181,6 +254,21 @@ struct Group {
         for (int ww = 1; ww < WARPS; ++ww) {
           s += buf[ww * 2];
           f |= (unsigned)__double2loint(buf[ww * 2 + 1]);
+        }
+        if constexpr (CL > 1) {   // the flag word rides as the low half of a double (OR-folded, never added)
+          double* xb = red + 2 * WARPS * 8 + parity * 8;
+          if (threadIdx.x == 0) {
+            xb[0] = s;
+            xb[1] = __hiloint2double(0, (int)f);
+          }
+          cluster_sync();
+          s = ld_dsmem(xb, 0u);
+          f = (unsigned)__double2loint(ld_dsmem(xb + 1, 0u));
+#pragma unroll
+          for (int r = 1; r < CL; ++r) {
+            s += ld_dsmem(xb, (uint32_t)r);
+            f |= (unsigned)__double2loint(ld_dsmem(xb + 1, (uint32_t)r));
+          }
         }
         x = s;
         flags = f;
@@ -217,9 +305,19 @@ struct Group {
           for (int ww = 1; ww < WARPS; ++ww) s = maxn2(s, buf[ww * NV + k]);
           x[k] = s;
         }
+        if constexpr (CL > 1) cluster_fold<NV>(x, red, parity, MaxN());
         parity ^= 1;
       }
     }
+  }
+
+  // OR of a predicate over a cluster group (CL > 1): CTA vote, then the CTAs' votes folded like a sum
+  __device__ __forceinline__ static bool any_cluster(bool p, double* red, int& parity) {
+    static_assert(CL > 1, "any_cluster: a group that spans a cluster");
+    double x[1] = {__syncthreads_or(p) ? 1.0 : 0.0};
+    cluster_fold<1>(x, red, parity, Plus());
+    parity ^= 1;
+    return x[0] != 0.0;
   }
 
   // broadcast a value chosen by thread 0 of the group (used for queue grabs)
@@ -228,6 +326,14 @@ struct Group {
       return v;
     } else if constexpr (G <= 32) {
       return __shfl_sync(mask(), v, (threadIdx.x & 31u) & ~(unsigned)(G - 1));
+    } else if constexpr (CL > 1) {
+      // thread 0 of rank 0 chose v; every CTA reads it from rank 0's shared memory.  The first barrier orders this
+      // write after every read of the previous broadcast -- and, at the first call of the kernel, after every CTA of
+      // the cluster has started (no DSMEM access reaches a CTA that is not running).
+      cluster_sync();
+      if (threadIdx.x == 0 && cluster_rank() == 0u) *sh = v;
+      cluster_sync();
+      return ld_dsmem(sh, 0u);
     } else {
       __syncthreads();
       if (threadIdx.x == 0) *sh = v;

@@ -81,6 +81,17 @@ static bool pick_generic(int d, LaunchPlan& p) {
   WN_PICK(64, 8, 64)
   WN_PICK(256, 4, 256)
   WN_PICK(512, 4, 512)     // d <= 4096: one 16-warp CTA per chain, one CTA per SM
+  // d <= 8192 / 16384 / 32768: one chain per thread-block CLUSTER of 2 / 4 / 8 such CTAs (G > NT), the reductions
+  // finished through distributed shared memory.  Package mode stays at one CTA per chain.  Measured on B200
+  // (scripts/high_d_gauss.py, profiles/r03_high_d_gauss.txt): see DESIGN.md section 2.  At 512 threads the register cap
+  // is 128, and ptxas spills a little (ptxas -v: 8-144 B of spill stores in the wpy / nuts / adapt kernels, about
+  // 1-1.8 KB in the ext kernels, whose extra integrators are not a hot path) -- the same as the 512 x 4 one-CTA rows
+  // above, which share the shape.  Other shapes (256 threads per CTA, 2 CTAs per SM) were not measured.
+  if constexpr (FAM != FAM_PKG) {
+    WN_PICK(1024, 4, 512)
+    WN_PICK(2048, 4, 512)
+    WN_PICK(4096, 4, 512)
+  }
   return false;
 }
 // targets that need the chain inside one warp; FIRST = false leaves out the first row for a caller that serves those d

@@ -37,6 +37,7 @@ struct wn_handle {
   float last_ms = 0.f;
   int64_t last_launches = 0;
   int32_t last_plan[4] = {-1, 0, 0, 0};   // {WN_FAMILY_*, G, E2, NT} of the last launch (wn_last_plan)
+  int64_t last_slots = 0;                  // chain slots of the last launch (wn_last_slots)
   unsigned long long last_tot[2] = {0, 0};
   int num_sms = 148;
   // grow-only device staging of the host-buffer paths (wn_run / wn_run_stats / wn_run_host_async)

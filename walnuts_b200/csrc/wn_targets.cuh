@@ -34,8 +34,8 @@ struct DiagGaussT {
   static constexpr bool PAIR_LAYOUT = true;
   static constexpr bool BLOCK_LOCKSTEP = false;
   // Energies are only consumed at the end of a pass (adaptiveIntegrators.py:87) plus the
-  // all(isfinite(Hams)) test (:92).  While every |q_i|, |v_i| stays below 2^470 (and inv_var <= 2^60, d <= 2^11 per
-  // chain group) each intermediate energy -- every term AND their sum -- is provably finite, so the intermediate
+  // all(isfinite(Hams)) test (:92).  While every |q_i|, |v_i| stays below 2^470 (and inv_var <= 2^60, d < 2^23; the
+  // dispatcher stops at d = 2^15) each intermediate energy -- every term AND their sum -- is provably finite, so the intermediate
   // steps may skip the two energy FMAs per
   // coordinate; if the bound is ever violated the sampler re-runs the pass with per-step energies.
   static constexpr bool LAZY_ENERGY = true;

@@ -135,21 +135,32 @@ __host__ __device__ constexpr int wpy_smem_doubles() {
   using Target = TargetTT<G, E2>;
   constexpr bool NF = NutsFast<Target, G, ADAPT, KSET>::value;
   return (NF ? 2 * NutsCfg<G, E2, NT>::NSM : 3) * 2 * E2 * NT + (NF ? 2 * NT : 0) +
-         2 * ((G + 31) / 32) * 8 + Target::smem_doubles(NT);
+         Group<G, (G > NT) ? NT : G>::RED_DOUBLES + Target::smem_doubles(NT);
 }
 
 // CTLSM: the cold control block of chains that SHARE a warp (G < 32) lives in shared memory (one copy per chain)
 // instead of per-thread registers / local memory -- fewer registers, more resident warps (G >= 32 always does).
+// G > NT: one chain per thread-block CLUSTER of CL = G / NT CTAs (launched with the cluster dimension CL); thread t of
+// the chain group is thread threadIdx.x of cluster rank t / NT.  Everything per chain that lives in shared memory
+// (control block, checkpoint, left-end slots, uniform buffer) is replicated or split per CTA exactly as for a
+// one-CTA group; only the Group<G, NT> reductions, the pass-end vote, the adaptation history and the queue grab cross
+// CTAs.
 template <template <int, int> class TargetTT, int G, int E2, int NT, int MINB = 1, bool ADAPT = false, bool EXT = false,
           int KSET = KSET_ANY, bool CTLSM = false>
 __global__ void __launch_bounds__(NT, MINB) walnutspy_kernel(const __grid_constant__ RunParams P) {
   static_assert(!EXT || ADAPT, "EXT kernels are built with the adaptation code (inactive without wn_set_adapt)");
   static_assert(KSET == KSET_ANY || (!ADAPT && !EXT), "specialised kernel sets exist for the plain family only");
   constexpr int E = 2 * E2;
-  constexpr int GPB = NT / G;  // groups per block
-  static_assert(NT % G == 0 && (G <= 32 || NT == G), "block must hold whole groups");
-  using Grp = Group<G>;
+  constexpr int GPB = NT / G;  // groups per block (0 for a cluster group: unused there)
+  static_assert((G <= NT) ? (NT % G == 0 && (G <= 32 || NT == G))
+                          : (G % NT == 0 && NT % 32 == 0 && (G / NT == 2 || G / NT == 4 || G / NT == 8)),
+                "block must hold whole groups, or a cluster of 2, 4 or 8 blocks one group");
+  // Grp::CL: CTAs per chain.  (Read from the group type, not declared as a local constant: an extra constexpr local
+  // changed the code ptxas emits for some existing kernels.)
+  using Grp = Group<G, (G > NT) ? NT : G>;
   using Target = TargetTT<G, E2>;
+  static_assert(Grp::CL == 1 || (!Target::COOP && !Target::BLOCK_LOCKSTEP),
+                "block-cooperative and lock-stepped targets need every chain of a block inside that block");
   constexpr bool NUTS_FAST = NutsFast<Target, G, ADAPT, KSET>::value;
   constexpr int NSM = NutsCfg<G, E2, NT>::NSM;
   constexpr bool LAZY = Target::LAZY_ENERGY && KSET != KSET_FIXED;   // plain NUTS consumes every step's energy
@@ -161,7 +172,7 @@ __global__ void __launch_bounds__(NT, MINB) walnutspy_kernel(const __grid_consta
   extern __shared__ __align__(16) double smem[];
   double* ck = smem;                       // checkpoint: [3*E][NT]  (NUTS_FAST: left-end slots [NSM][2][E][NT])
   double* ubuf = smem + (NUTS_FAST ? 2 * NSM : 3) * E * NT;   // NUTS_FAST: buffered sequential uniforms, 2 per thread
-  double* red = ubuf + (NUTS_FAST ? 2 * NT : 0);              // reduction scratch (G > 32)
+  double* red = ubuf + (NUTS_FAST ? 2 * NT : 0);              // reduction scratch (G > 32; Grp::RED_DOUBLES)
   __shared__ uint32_t sh_bcast;
   constexpr bool CTL_SHARED = (G >= 32) || CTLSM;
   __shared__ Ctl sh_ctl[(G >= 32) ? NT / 32 : (CTLSM ? NT / G : 1)];
@@ -175,18 +186,19 @@ __global__ void __launch_bounds__(NT, MINB) walnutspy_kernel(const __grid_consta
   volatile int* ktab = sh_ktab[(G >= 32) ? (threadIdx.x >> 5) : 0];
 
   const int tid = threadIdx.x;
-  const int t = tid % G;
+  const int t = (Grp::CL > 1) ? (int)cluster_rank() * NT + tid : tid % G;
   int parity = 0;
 
-  // scratch addressing: vector vi, pair e2 -> scratch[((vi*E2 + e2) * nslot + slot) * G + t]
+  // scratch addressing: vector vi, pair e2 -> scratch[((vi*E2 + e2) * nslot + slot) * G + t]; slot = chain group
+  // (a cluster when G > NT: the grid is 1-D, so cluster c is blocks c CL .. c CL + CL - 1)
   // (computed on demand: a hoisted base pointer + stride would cost four live registers in the hot loop)
   auto sc = [&](int vi, int e2) -> double2* {
-    const size_t slot = (size_t)blockIdx.x * GPB + tid / G;
+    const size_t slot = (Grp::CL > 1) ? (size_t)(blockIdx.x / Grp::CL) : (size_t)blockIdx.x * GPB + tid / G;
     return P.scratch + ((size_t)(vi * E2 + e2) * P.nslot + slot) * G + t;
   };
 
   Target target;
-  target.init(P.tp, P.d, t, red + 2 * ((G + 31) / 32) * 8);
+  target.init(P.tp, P.d, t, red + Grp::RED_DOUBLES);
 
   // ---- register-resident working state -----------------------------------------------------
   double q[E], v[E], g[E];
@@ -215,20 +227,22 @@ __global__ void __launch_bounds__(NT, MINB) walnutspy_kernel(const __grid_consta
 
   // sequential scalar stream (STREAM_SEQ), draw n of the current iteration.  NUTS_FAST: the stream is counter-based,
   // so the group computes 2 G draws ahead at once (every thread one Philox block) into a shared buffer; a draw is
-  // then one shared load instead of ten Philox rounds replicated by every warp of the chain.
+  // then one shared load instead of ten Philox rounds replicated by every warp of the chain.  A cluster group: every
+  // CTA fills its own buffer with the same 2 NT draws (no DSMEM traffic, no cluster barrier).
   uint4 ublk = make_uint4(0u, 0u, 0u, 0u);
   uint32_t ublk_idx = 0xffffffffu;
   auto ufetch = [&](uint32_t n) -> double {
     RngKey key{P.seed_lo, P.seed_hi, C.chain, C.iter};
     if constexpr (NUTS_FAST) {
-      constexpr uint32_t UB = 2u * G;
-      double* ub = ubuf + (tid / G) * UB;
+      constexpr uint32_t UB = 2u * ((Grp::CL > 1) ? NT : G);
+      double* ub = ubuf + ((Grp::CL > 1) ? 0 : (tid / G) * UB);
+      const int ut = (Grp::CL > 1) ? tid : t;   // this thread's Philox block within the buffer
       if ((n % UB) == 0u) {
         if constexpr (G > 32) __syncthreads(); else __syncwarp();
         double u0, u1;
-        rng_uniform_pair(key, STREAM_SEQ, (n >> 1) + (uint32_t)t, u0, u1);
-        ub[2 * t] = u0;
-        ub[2 * t + 1] = u1;
+        rng_uniform_pair(key, STREAM_SEQ, (n >> 1) + (uint32_t)ut, u0, u1);
+        ub[2 * ut] = u0;
+        ub[2 * ut + 1] = u1;
         if constexpr (G > 32) __syncthreads(); else __syncwarp();
       }
       return ub[n % UB];
@@ -379,7 +393,9 @@ __global__ void __launch_bounds__(NT, MINB) walnutspy_kernel(const __grid_consta
         since = 0;
         // One leapfrog step amplifies max(|q|,|v|) by at most Gamma (target-specific bound); checked states are
         // below 2^300, so up to floor(170 / log2 Gamma) steps may pass between checks while every skipped energy
-        // stays finite: magnitudes < 2^470, terms q^2 s < 2^(940 + 60), their sum over d <= 2^11 coordinates < 2^1011.  Gamma grows with the step, so the interval is tabulated per c once per
+        // stays finite: magnitudes < 2^470, terms q^2 s and v^2 < 2^(940 + 60), so their sum over d <= 2^15
+        // coordinates (the largest dispatched) is < 2^1016 -- and below 2^1024 for any d < 2^23.  Gamma grows with
+        // the step, so the interval is tabulated per c once per
         // iteration for the LARGEST jittered macro step (ST_ITER: ktab), a conservative bound for every macro step.
         if constexpr (G >= 32) {
           lazyK = ktab[cc];
@@ -472,6 +488,9 @@ __global__ void __launch_bounds__(NT, MINB) walnutspy_kernel(const __grid_consta
 
   uint32_t coop_phase = 0;   // COOP targets: phase bits of the staging mbarriers
   int st = ST_CHAIN;
+  // cluster group: no CTA reads a peer's shared memory before the peer runs (the first DSMEM access, in the first
+  // queue grab, follows this barrier)
+  if constexpr (Grp::CL > 1) cluster_sync();
   // ===================== plain NUTS (fixedLeapFrog), whole warps per chain: one doubling level ======================
   // Replaces ST_MACRO -> ST_RUN -> ST_PASS_END -> ST_LEAF of the flat loop for the n_new = 2^level leaves of a level
   // (reference WALNUTS.py:296-368 for level 0, :392-587 for the leaf pairs; adaptiveIntegrators.py:49-59 per leaf).
@@ -836,7 +855,9 @@ __global__ void __launch_bounds__(NT, MINB) walnutspy_kernel(const __grid_consta
         if (rsearch && rc < rlim && target.nonneg_ok) {
           const bool lf = (hp > rHref) && (fabs(rHref - hp) >= rdelta);
           bool anyf;
-          if constexpr (G > 32) anyf = __syncthreads_or(lf) != 0;
+          // a cluster group votes over all its CTAs: the failing partial may sit in any of them
+          if constexpr (Grp::CL > 1) anyf = Grp::any_cluster(lf, red, parity);
+          else if constexpr (G > 32) anyf = __syncthreads_or(lf) != 0;
           else if constexpr (G > 1) anyf = __any_sync(Grp::mask(), lf) != 0;
           else anyf = lf;
           if (anyf) {
@@ -1208,12 +1229,15 @@ __global__ void __launch_bounds__(NT, MINB) walnutspy_kernel(const __grid_consta
               }
               newdelta = P.adTarget / qv;
             }
-            if constexpr (G > 32) __syncthreads(); else if constexpr (G > 1) __syncwarp(Grp::mask());
+            // every thread has read the row before thread 0 rewrites it, and sees the new row afterwards; a cluster
+            // group's row is read by the other CTAs, so both barriers are cluster barriers (release / acquire at
+            // cluster scope order the global-memory row as well)
+            if constexpr (Grp::CL > 1) cluster_sync(); else if constexpr (G > 32) __syncthreads(); else if constexpr (G > 1) __syncwarp(Grp::mask());
             if (t == 0 && fac == fac) {           // shift the tail and insert
               for (int i = n0; i > pos; --i) hrow[i] = hrow[i - 1];
               hrow[pos] = fac;
             }
-            if constexpr (G > 32) __syncthreads(); else if constexpr (G > 1) __syncwarp(Grp::mask());
+            if constexpr (Grp::CL > 1) cluster_sync(); else if constexpr (G > 32) __syncthreads(); else if constexpr (G > 1) __syncwarp(Grp::mask());
             C.adNhist = n1;
             delta = newdelta;
             C.delta = delta;
@@ -1252,6 +1276,8 @@ __global__ void __launch_bounds__(NT, MINB) walnutspy_kernel(const __grid_consta
       break;
     } while (0);
     if (st == ST_CHAIN) do {  // grab the next chain from the queue
+      // (cluster group: thread 0 of rank 0 grabs, bcast0 hands the SAME index to every CTA, so all CTAs of the cluster
+      // serve the same chain and leave the loop at the same trip -- every cluster barrier is reached by all of them)
       uint32_t cidx = 0;
       if (t == 0) {
         cidx = atomicAdd(P.queue, 1u);
@@ -1735,6 +1761,9 @@ __global__ void __launch_bounds__(NT, MINB) walnutspy_kernel(const __grid_consta
       break;
     }
   }
+  // cluster group: no CTA exits while a peer may still read its shared memory (the last DSMEM access is the exit
+  // grab's broadcast, which every CTA passed before leaving the loop at the same trip)
+  if constexpr (Grp::CL > 1) cluster_sync();
   if (t == 0 && (totF | totB)) {
     atomicAdd(P.totals, totF);
     atomicAdd(P.totals + 1, totB);

@@ -220,10 +220,17 @@ class ChainBatch:
 
     def last_plan(self):
         """(family, G, E2, NT) of the last run: the kernel family (_ffi.FAMILIES), threads per chain, coordinate pairs
-        per thread and threads per block; family -1 before the first run."""
+        per thread and threads per block; family -1 before the first run.  G > NT: each chain runs on a thread-block
+        cluster of G / NT blocks."""
         out = (C.c_int32 * 4)()
         self._check(self._lib.wn_last_plan(self._h, out), "wn_last_plan")
         return tuple(int(x) for x in out)
+
+    def last_slots(self):
+        """Chain slots of the last run: chain groups resident at once (clusters when G > NT), at most n_chains."""
+        n = C.c_int64()
+        self._check(self._lib.wn_last_slots(self._h, C.byref(n)), "wn_last_slots")
+        return int(n.value)
 
     def last_grad_evals(self):
         f, b = C.c_uint64(), C.c_uint64()
