@@ -77,27 +77,89 @@ def logreg(X, y, tau=1.0):
     return Target("logreg", data={"X": X, "y": y, "tau": np.array([float(tau)])}, d=X.shape[1], ref="SURVEY.md T4")
 
 
-def cuda_target(source, d, data=None, name="user", verbose=False):
+# Parallel protocol plans (wn_user_plugin.cuh, UserParT): (largest d, threads per chain G, coordinate pairs per thread
+# E2, threads per block NT) -- the shapes the built-in targets run on (wn_dispatch.cuh: pick_generic)
+PARALLEL_PLANS = [(256, 32, 4, 128), (512, 32, 8, 128), (1024, 64, 8, 64), (2048, 256, 4, 256), (4096, 512, 4, 512)]
+SMEM_MAX = 227 * 1024          # shared memory of one block on sm_100a
+_CTL_BYTES = 504               # sizeof(wn::Ctl), the per-warp control block of walnutspy_kernel
+
+
+def parallel_plan(d):
+    """(G, E2, NT) of a parallel-protocol user target of dimension d."""
+    for dmax, G, E2, NT in PARALLEL_PLANS:
+        if d <= dmax:
+            return G, E2, NT
+    raise ValueError(f"cuda_target(parallel=True): 1 <= d <= {PARALLEL_PLANS[-1][0]}")
+
+
+def parallel_smem_bytes(d, scratch):
+    """Shared memory per block of a parallel user target's kernels in bytes: the larger of the WALNUTSpy (EXT) and
+    package kernels, dynamic part plus static arrays, computed as the plug-in's static_assert computes it."""
+    G, E2, NT = parallel_plan(d)
+    r16 = lambda b: (b + 15) // 16 * 16
+    w = NT // 32
+    dyn = 3 * 2 * E2 * NT + 2 * ((G + 31) // 32) * 8 + (NT // G) * (2 * 2 * G * E2 + scratch)
+    # the package kernel has the same dynamic part and a smaller static one (its control block is smaller, no table)
+    return 8 * dyn + r16(4) + r16(_CTL_BYTES * w) + r16(4 * 32 * w)
+
+
+def cuda_target(source, d, data=None, name="user", verbose=False, *, parallel=False, scratch=0):
     """A user-defined target: the role of the reference's arbitrary Python `lpFun` (WALNUTSpy/targetDistr.py:18) /
     `logp`, `grad` (walnuts/walnuts.py:296-297) callables and of walnuts_stan.py's compiled Stan model.
 
-    `source` is CUDA C++ defining the log density and its gradient over the whole coordinate vector:
+    Sequential protocol (parallel=False, 1 <= d <= 512): `source` is CUDA C++ defining the log density and its
+    gradient over the whole coordinate vector:
 
         WN_TARGET_LP_GRAD(q, g, data, n_data) {
             // q[0..WN_D-1] in, g[0..WN_D-1] out; data[0..n_data-1] is the `data` array; return the log density
         }
 
+    d <= 64 runs one thread per chain; 64 < d <= 512 one warp per chain -- leapfrog and tree logic parallel over the
+    lanes, the user's function evaluated by every lane on the whole vector.
+
+    Parallel protocol (parallel=True, 1 <= d <= 4096): every thread of the chain's group (32 threads for d <= 512, 64
+    for d <= 1024, 256 for d <= 2048, 512 for d <= 4096) calls the function at once and computes its share:
+
+        WN_TARGET_LP_GRAD_PAR(q, g, data, n_data, ctx) {
+            // q[0..WN_D-1]: the chain's position in shared memory, readable by every thread of the chain
+            for (int j = ctx.rank; j < WN_D; j += ctx.size) g[j] = ...;   // the gradient entries this thread owns
+            // ctx.sum(x): sum over the chain's threads (same value on every thread); ctx.sync(): barrier over them;
+            // ctx.scratch: `scratch` doubles of per-chain shared memory
+            return share;   // this thread's share of lp; the library adds the shares
+        }
+
+    Every thread of the chain must call ctx.sum and ctx.sync the same number of times in the same order (a call in a
+    branch that differs between threads is undefined behaviour); indices j >= d are never handed out.  `scratch` is
+    limited by the 227 KB of shared memory of a block (parallel_smem_bytes).  Defining the macro of the other protocol
+    fails to compile with a message naming the right one.
+
     It is compiled once with nvcc for sm_100a into walnuts_b200/_lib/user/<hash>.so (cached by content), linked
-    against the same persistent kernels as the built-in targets (d <= 64: one thread per chain; 64 < d <= 512: one warp
-    per chain -- leapfrog and tree logic parallel over the lanes, the user's function evaluated on the whole vector), and serves
-    WALNUTS(...) with every integrator and the warm-up adaptation as well as walnuts(...) / walnuts_step(...)."""
+    against the same persistent kernels as the built-in targets, and serves WALNUTS(...) with every integrator and the
+    warm-up adaptation as well as walnuts(...) / walnuts_step(...)."""
     from . import build as _build
     d = int(d)
-    if not 1 <= d <= 512:
-        raise ValueError("cuda_target: 1 <= d <= 512 (d <= 64: one thread per chain holds the whole vector; "
-                         "64 < d <= 512: one warp per chain, the density evaluated by every lane on the whole vector)")
+    scratch = int(scratch)
+    if parallel:
+        if not 1 <= d <= PARALLEL_PLANS[-1][0]:
+            raise ValueError(f"cuda_target(parallel=True): 1 <= d <= {PARALLEL_PLANS[-1][0]} (one chain per warp up to "
+                             "d = 512, per block of 64 / 256 / 512 threads up to d = 1024 / 2048 / 4096)")
+        if scratch < 0:
+            raise ValueError("cuda_target: scratch must be >= 0 doubles")
+        need = parallel_smem_bytes(d, scratch)
+        if need > SMEM_MAX:
+            raise ValueError(f"cuda_target: scratch={scratch} needs {need} bytes of shared memory per block at d = {d}, "
+                             f"more than the {SMEM_MAX} of a block")
+    else:
+        if scratch != 0:
+            raise ValueError("cuda_target: scratch needs parallel=True")
+        if not 1 <= d <= 512:
+            raise ValueError("cuda_target: 1 <= d <= 512 (d <= 64: one thread per chain holds the whole vector; "
+                             "64 < d <= 512: one warp per chain, the density evaluated by every lane on the whole vector)")
     csrc = os.path.join(_build.HERE, "csrc")
-    tu = (f"#define WN_USER_D {d}\n#include \"wn_user_api.cuh\"\n#line 1 \"{name}\"\n{source}\n"
+    head = f"#define WN_USER_D {d}\n"
+    if parallel:
+        head += f"#define WN_USER_PARALLEL 1\n#define WN_USER_SCRATCH {scratch}\n"
+    tu = (f"{head}#include \"wn_user_api.cuh\"\n#line 1 \"{name}\"\n{source}\n"
           "#include \"wn_user_plugin.cuh\"\n")
     h = hashlib.sha256()
     h.update(tu.encode())
