@@ -217,6 +217,45 @@ int wn_comm_destroy(wn_handle* h);
 int wn_ess_rhat(wn_handle* h, const double* draws, int64_t n_iter, int64_t n_chains, int32_t dg, int on_device,
                 int32_t split, double* ess, double* rhat);
 
+/* Posterior summary per monitored coordinate, computed on the device: out is a host array [dg][WN_SUMMARY_COLS] with
+ * the columns below.  Draws, limits (n_iter >= 4, <= 25 600 draws per split chain, <= 2^31 draws per coordinate) and
+ * pooling are those of wn_ess_rhat: with a communicator the draws of all ranks are pooled by the same one all-gather,
+ * global chain order is rank-major (the devices= sharding order), and every rank receives the same result.
+ * superchain_size = 0: no nested R-hat (that column is NaN).  s > 0: global chains k*s ... k*s + s - 1 form superchain k;
+ * the chain count over all ranks must be a multiple of s with at least 2 superchains, else WN_EINVAL.
+ *
+ * Definitions for one coordinate: x has M chains x N draws, S = M N.  "Split ESS of y" splits every chain of y into
+ * [0, h) and [N - h, N), h = N / 2, and applies the estimator of wn_ess_rhat WITHOUT rank normalisation.
+ *   WN_S_MEAN, WN_S_SD          mean and sd over all S draws; sd with 1 / (S - 1)
+ *   WN_S_Q05, _Q50, _Q95        linear-interpolation quantiles (numpy's default) of the S sorted draws
+ *   WN_S_MCSE_MEAN              sd / sqrt(split ESS of x)
+ *   WN_S_MCSE_SD                c = (x - mean)^2, E = mean(c), varvar = (mean(c^2) - E^2) / split ESS of c,
+ *                               sqrt(varvar / (4 E))
+ *   WN_S_ESS_BULK               the ess of wn_ess_rhat with split = 1, bit for bit
+ *   WN_S_ESS_TAIL               min(split ESS of 1[x <= q05], split ESS of 1[x <= q95]); indicators not rank-normalised
+ *   WN_S_RHAT                   max(the rhat of wn_ess_rhat with split = 1, the same R-hat of |x - q50|)
+ *   WN_S_NESTED_RHAT            sqrt(1 + B / W) on the raw draws (Margossian, Hoffman, Sountsov, Riou-Durand, Vehtari,
+ *                               Gelman 2024): B = 1/(K-1) sum_k (xbar_k - xbar)^2 over the K superchain means,
+ *                               W = 1/K sum_k (Btilde_k + Wtilde_k), Btilde_k = 1/(s-1) sum_m (xbar_mk - xbar_k)^2
+ *                               (0 for s = 1), Wtilde_k = 1/s sum_m (within-chain variance with 1 / (N - 1))
+ * Conventions, as wn_ess_rhat: ranks are ordinal (ties broken by chain-major position) and taken over all S draws
+ * before the split, so for odd N the middle draw is ranked but dropped; an ESS or R-hat of a series with zero variance
+ * is NaN, and so is every column computed from one (min and max are NaN when either argument is). */
+#define WN_SUMMARY_COLS 11
+#define WN_S_MEAN 0
+#define WN_S_SD 1
+#define WN_S_Q05 2
+#define WN_S_Q50 3
+#define WN_S_Q95 4
+#define WN_S_MCSE_MEAN 5
+#define WN_S_MCSE_SD 6
+#define WN_S_ESS_BULK 7
+#define WN_S_ESS_TAIL 8
+#define WN_S_RHAT 9
+#define WN_S_NESTED_RHAT 10
+int wn_summary(wn_handle* h, const double* draws, int64_t n_iter, int64_t n_chains, int32_t dg, int on_device,
+               int32_t superchain_size, double* out);
+
 /* wn_moments over the chains of ALL ranks of the communicator (two all-reduces of d + 1 doubles). */
 int wn_moments_all(wn_handle* h, double* mean, double* var);
 

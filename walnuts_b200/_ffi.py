@@ -10,6 +10,8 @@ MODE_WALNUTSPY, MODE_PACKAGE = 0, 1
 INT_FIXED, INT_D, INT_R2P = 0, 1, 2
 DIAG_COLS = 24
 FAMILIES = {"wpy": 0, "pkg": 1, "adapt": 2, "ext": 3, "nuts": 4}      # WN_FAMILY_* (wn_last_plan)
+# WN_S_* columns of wn_summary, in order
+SUMMARY_COLS = ("mean", "sd", "q05", "q50", "q95", "mcse_mean", "mcse_sd", "ess_bulk", "ess_tail", "rhat", "nested_rhat")
 ERRORS = {-1: "WN_EINVAL", -2: "WN_ECUDA", -3: "WN_ENOMEM", -4: "WN_EUNSUPPORTED", -5: "WN_ESTATE"}
 
 # every symbol include/walnuts_cuda.h declares
@@ -17,7 +19,7 @@ SYMBOLS = ["wn_abi_version", "wn_target_id", "wn_register_user_target", "wn_crea
            "wn_get_state", "wn_run", "wn_run_stats", "wn_run_async", "wn_sync", "wn_run_host_async", "wn_alloc_pinned", "wn_free_pinned", "wn_last_kernel_ms", "wn_last_launches",
            "wn_last_plan", "wn_last_slots", "wn_last_grad_evals", "wn_moments", "wn_stream", "wn_last_error", "wn_fp64_peak",
            "wn_comm_load", "wn_comm_unique_id", "wn_comm_init_rank", "wn_comm_init_all", "wn_comm_destroy",
-           "wn_ess_rhat", "wn_moments_all"]
+           "wn_ess_rhat", "wn_summary", "wn_moments_all"]
 
 
 class WnConfig(C.Structure):
@@ -82,6 +84,7 @@ def load():
     lib.wn_comm_init_all.argtypes = [P(vp), C.c_int]
     lib.wn_comm_destroy.argtypes = [vp]
     lib.wn_ess_rhat.argtypes = [vp, dp, C.c_int64, C.c_int64, C.c_int32, C.c_int, C.c_int32, dp, dp]
+    lib.wn_summary.argtypes = [vp, dp, C.c_int64, C.c_int64, C.c_int32, C.c_int, C.c_int32, dp]
     lib.wn_moments_all.argtypes = [vp, dp, dp]
     lib.wn_stream.argtypes = [vp]
     lib.wn_stream.restype = vp

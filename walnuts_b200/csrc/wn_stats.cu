@@ -10,6 +10,14 @@
 // Pipeline of wn_ess_rhat per coordinate: gather column -> radix sort (cub) -> ranks -> z = Phi^-1((r - 3/8) / (S + 1/4))
 // -> split every chain in halves -> per split chain: mean, variance and ALL autocovariances in shared memory -> sums over
 // chains in a fixed order -> Geyer's initial monotone sequence on the host (a few thousand numbers).
+//
+// wn_summary runs the same pipeline per coordinate (its bulk ESS and R-hat are the same bits), then reads the quantiles
+// and moments from the sorted column (summary_moments), feeds the raw draws, the two tail indicators and the squared
+// deviations through the same split-chain sums, and ranks |x - q50| with a second radix sort.  The second sort rather
+// than a merge of the two halves of the sorted column around the median: |x - q50| is rounded, so distinct draws can
+// fold to the same value, and ordinal ranks then follow the chain-major position, which the merge does not see; the
+// sort gives the ranks the definition asks for in every case.  Nested R-hat: chain moments, one warp per chain, then
+// one block over the superchains.  One host synchronisation per coordinate, as in wn_ess_rhat.
 #include <dlfcn.h>
 #include <nccl.h>   // types and enums only; every function is resolved with dlsym
 
@@ -144,6 +152,156 @@ __global__ void reduce_chains(const double* __restrict__ acov, const double* __r
   }
 }
 
+// ---- posterior summary (wn_summary) ----
+
+// Sum of one value per thread over the block in a fixed order (shuffle tree per warp, then the warps in order); every
+// thread receives the sum.  blockDim.x is a multiple of 32; red holds 32 doubles of shared memory.
+__device__ double block_sum(double v, double* red) {
+  for (int o = 16; o >= 1; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  __syncthreads();   // red may still be read from the previous call
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  double t = 0.0;
+  for (int w = 0; w < (int)(blockDim.x >> 5); ++w) t += red[w];
+  return t;
+}
+
+// numpy's default ('linear') quantile p of the sorted xs[0, S): v = (S - 1) p, a = xs[floor v], b = the next draw,
+// t = v - floor v, then a + (b - a) t for t < 1/2 and b - (b - a)(1 - t) otherwise, rounded as numpy rounds it (no FMA)
+__device__ double quantile_sorted(const double* __restrict__ xs, size_t S, double p) {
+  const double v = __dmul_rn((double)(S - 1), p);
+  if (v >= (double)(S - 1)) return xs[S - 1];
+  const double f = floor(v);
+  const size_t i = (size_t)f;
+  const double a = xs[i], b = xs[i + 1], t = v - f, d = b - a;
+  return t >= 0.5 ? __dsub_rn(b, __dmul_rn(d, 1.0 - t)) : __dadd_rn(a, __dmul_rn(d, t));
+}
+
+// Quantiles and central moments of one coordinate from its sorted draws xs[0, S), in a fixed order: the same bits on
+// every run and for every rank count, because every rank sorts the same pooled column.  Each block sums the powers
+// 1..4 of d = x - q50 over a fixed grid-stride set of draws; the last block to finish adds the partials in block order
+// and writes sc = {mean, q05, q50, q95, sum (x - mean)^2, sum (x - mean)^4}.  Centring at the median keeps the power
+// sums well conditioned (|mean - median| <= sd).  *done is 0 on entry and is left 0.
+__global__ void summary_moments(const double* __restrict__ xs, size_t S, double* __restrict__ part,
+                                unsigned* __restrict__ done, double* __restrict__ sc) {
+  __shared__ double red[32];
+  __shared__ bool last;
+  const double q50 = quantile_sorted(xs, S, 0.5);
+  double p1 = 0.0, p2 = 0.0, p3 = 0.0, p4 = 0.0;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < S; i += (size_t)gridDim.x * blockDim.x) {
+    const double d = xs[i] - q50, d2 = d * d;
+    p1 += d;
+    p2 += d2;
+    p3 = fma(d2, d, p3);
+    p4 = fma(d2, d2, p4);
+  }
+  p1 = block_sum(p1, red);
+  p2 = block_sum(p2, red);
+  p3 = block_sum(p3, red);
+  p4 = block_sum(p4, red);
+  if (threadIdx.x == 0) {
+    double* pb = part + 4 * (size_t)blockIdx.x;
+    pb[0] = p1; pb[1] = p2; pb[2] = p3; pb[3] = p4;
+    __threadfence();   // the partials are visible to the last block before it counts this one
+    last = atomicAdd(done, 1u) == gridDim.x - 1;
+  }
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  double s1 = 0.0, s2 = 0.0, s3 = 0.0, s4 = 0.0;
+  for (int b = threadIdx.x; b < (int)gridDim.x; b += blockDim.x) {
+    const double* pb = part + 4 * (size_t)b;
+    s1 += __ldcg(pb); s2 += __ldcg(pb + 1); s3 += __ldcg(pb + 2); s4 += __ldcg(pb + 3);
+  }
+  s1 = block_sum(s1, red);
+  s2 = block_sum(s2, red);
+  s3 = block_sum(s3, red);
+  s4 = block_sum(s4, red);
+  if (threadIdx.x == 0) {
+    const double n = (double)S, e = s1 / n, e2 = e * e;   // e = mean - q50
+    sc[0] = q50 + e;
+    sc[1] = quantile_sorted(xs, S, 0.05);
+    sc[2] = q50;
+    sc[3] = quantile_sorted(xs, S, 0.95);
+    sc[4] = s2 - s1 * e;                                        // sum (d - e)^2
+    sc[5] = s4 - 4.0 * e * s3 + 6.0 * e2 * s2 - 3.0 * n * e2 * e2;   // sum (d - e)^4
+    *done = 0u;
+  }
+}
+
+// The series of one coordinate whose split-chain statistics the summary needs, element-wise from the chain-major
+// column x and sc (summary_moments): kind 0: 1[x <= q05], 1: 1[x <= q95], 2: (x - mean)^2, 3: |x - q50|
+__global__ void summary_series(const double* __restrict__ x, size_t S, const double* __restrict__ sc, int kind,
+                               double* __restrict__ y) {
+  const double mean = sc[0], q05 = sc[1], q50 = sc[2], q95 = sc[3];
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < S; i += (size_t)gridDim.x * blockDim.x) {
+    const double v = x[i];
+    double r;
+    if (kind == 0) r = v <= q05 ? 1.0 : 0.0;
+    else if (kind == 1) r = v <= q95 ? 1.0 : 0.0;
+    else if (kind == 2) r = (v - mean) * (v - mean);
+    else r = fabs(v - q50);
+    y[i] = r;
+  }
+}
+
+// Mean and variance (1 / (n - 1)) of every whole chain of the chain-major column x; one warp per chain, fixed order
+__global__ void chain_moments(const double* __restrict__ x, int n, int n_chains, double* __restrict__ mean,
+                              double* __restrict__ var) {
+  const int c = (int)(((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+  if (c >= n_chains) return;   // c is uniform over the warp
+  const double* v = x + (size_t)c * n;
+  double s = 0.0;
+  for (int i = lane; i < n; i += 32) s += v[i];
+  for (int o = 16; o >= 1; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  const double m = s / n;
+  double q = 0.0;
+  for (int i = lane; i < n; i += 32) {
+    const double d = v[i] - m;
+    q = fma(d, d, q);
+  }
+  for (int o = 16; o >= 1; o >>= 1) q += __shfl_xor_sync(0xffffffffu, q, o);
+  if (lane == 0) {
+    mean[c] = m;
+    var[c] = q / (n - 1);
+  }
+}
+
+// Nested R-hat of K superchains of s consecutive chains from the chain moments; one block, fixed order.
+// out = sqrt(1 + B / W), B = 1/(K-1) sum_k (xbar_k - xbar)^2, W = 1/K sum_k (Btilde_k + What_k) with
+// Btilde_k = 1/(s-1) sum_m (xbar_mk - xbar_k)^2 (0 for s = 1) and What_k = 1/s sum_m var_mk.
+__global__ void nested_rhat(const double* __restrict__ mean, const double* __restrict__ var, int K, int s,
+                            double* __restrict__ out) {
+  __shared__ double red[32];
+  auto super_mean = [&](int k) {
+    double a = 0.0;
+    for (int m = 0; m < s; ++m) a += mean[(size_t)k * s + m];
+    return a / s;
+  };
+  double a = 0.0, w = 0.0;
+  for (int k = threadIdx.x; k < K; k += blockDim.x) {
+    const double mk = super_mean(k);
+    double b = 0.0, v = 0.0;
+    for (int m = 0; m < s; ++m) {
+      const double e = mean[(size_t)k * s + m] - mk;
+      b = fma(e, e, b);
+      v += var[(size_t)k * s + m];
+    }
+    a += mk;
+    w += (s > 1 ? b / (s - 1) : 0.0) + v / s;
+  }
+  a = block_sum(a, red);
+  w = block_sum(w, red);
+  const double xbar = a / K;
+  double b = 0.0;
+  for (int k = threadIdx.x; k < K; k += blockDim.x) {
+    const double e = super_mean(k) - xbar;
+    b = fma(e, e, b);
+  }
+  b = block_sum(b, red);
+  if (threadIdx.x == 0) *out = sqrt(1.0 + (b / (K - 1)) / (w / K));
+}
+
 // out[j] = sum over chains of state[c][j]  (pass 1)  /  of (state[c][j] - mean[j])^2  (pass 2, mean != null)
 __global__ void moment_sums(const double* __restrict__ state, int n_chains, int d, const double* __restrict__ mean,
                             double* __restrict__ out) {
@@ -201,6 +359,94 @@ void ess_from_sums(const double* acov_sum, int T, int m, int n, double sum_mean,
   *ess = total / tau;
   *rhat = mean_var > 0 ? std::sqrt(var_plus / mean_var) : nan;
 }
+
+// Device buffers of one statistics call, freed when the call returns
+struct DevBufs {
+  std::vector<void*> ptrs;
+  ~DevBufs() {
+    for (void* p : ptrs) cudaFree(p);
+  }
+  template <class T>
+  cudaError_t alloc(T** out, size_t n) {
+    *out = nullptr;
+    const cudaError_t e = cudaMalloc((void**)out, n * sizeof(T));
+    if (e == cudaSuccess) ptrs.push_back(*out);
+    return e;
+  }
+};
+
+#define ST_TRY(expr)                                                                           \
+  do {                                                                                         \
+    const cudaError_t _e = (expr);                                                             \
+    if (_e != cudaSuccess) return fail(h, WN_ECUDA, std::string(#expr) + ": " + cudaGetErrorString(_e)); \
+  } while (0)
+
+// The draws of every rank on this device, [W][n_iter][n_chains][dg]: a copy of host draws, then the one all-gather of
+// a multi-GPU run (every rank receives the monitored draws of all chains).
+int pooled_draws(wn_handle* h, const double* draws, size_t per_rank, int on_device, DevBufs& bufs,
+                 const double** src) {
+  cudaStream_t st = h->stream;
+  *src = draws;
+  if (!on_device) {
+    double* d_in = nullptr;
+    ST_TRY(bufs.alloc(&d_in, per_rank));
+    ST_TRY(cudaMemcpyAsync(d_in, draws, per_rank * sizeof(double), cudaMemcpyHostToDevice, st));
+    *src = d_in;
+  }
+  if (h->comm) {
+    double* d_all = nullptr;
+    ST_TRY(bufs.alloc(&d_all, per_rank * h->comm_size));
+    const ncclResult_t r = g_nccl.AllGather(*src, d_all, per_rank, ncclDouble, (ncclComm_t)h->comm, st);
+    if (r != ncclSuccess) return fail(h, WN_ECUDA, std::string("ncclAllGather: ") + g_nccl.GetErrorString(r));
+    *src = d_all;
+  }
+  return WN_OK;
+}
+
+// The per-coordinate pipeline of wn_ess_rhat, which wn_summary runs too (so that its bulk ESS and R-hat are the same
+// bits): gather a column of the pooled draws, sort it, rank-normalise, split-chain sums.
+struct ColumnWork {
+  int W, n, n_chains, dg, hlen, split, n_split, nb;
+  size_t S;
+  cudaStream_t st;
+  double *x, *xs, *z, *mean, *var, *acov;
+  unsigned *idx, *idxs;
+  char* tmp = nullptr;
+  size_t tmp_bytes = 0;
+
+  ColumnWork(int W_, int n_, int n_chains_, int dg_, int split_, cudaStream_t st_)
+      : W(W_), n(n_), n_chains(n_chains_), dg(dg_), hlen(split_ ? n_ / 2 : n_), split(split_ ? 1 : 0),
+        n_split(W_ * n_chains_ * (split_ ? 2 : 1)), S((size_t)W_ * n_ * n_chains_), st(st_) {
+    nb = (int)((S + 255) / 256 < 4096 ? (S + 255) / 256 : 4096);
+  }
+  cudaError_t alloc(DevBufs& b) {
+    cudaError_t e;
+    if ((e = b.alloc(&x, S)) || (e = b.alloc(&xs, S)) || (e = b.alloc(&z, S)) || (e = b.alloc(&idx, S)) ||
+        (e = b.alloc(&idxs, S)) || (e = b.alloc(&mean, n_split)) || (e = b.alloc(&var, n_split)) ||
+        (e = b.alloc(&acov, (size_t)n_split * hlen)))
+      return e;
+    if ((e = cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, x, xs, idx, idxs, (int)S, 0, 64, st))) return e;
+    if ((e = b.alloc(&tmp, tmp_bytes))) return e;
+    return cudaFuncSetAttribute(split_chain_stats, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(hlen * sizeof(double)));
+  }
+  // column j of the pooled draws -> x (chain-major), idx = identity
+  void gather(const double* src, int j) { gather_column<<<nb, 256, 0, st>>>(src, W, n, n_chains, dg, j, x, idx); }
+  // keys (chain-major) sorted with idx into xs / idxs; z = the rank-normalised keys, chain-major.  idx stays identity.
+  cudaError_t sort_rank(const double* keys) {
+    const cudaError_t e = cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, xs, idx, idxs, (int)S, 0, 64, st);
+    if (e) return e;
+    rank_normalize<<<nb, 256, 0, st>>>(idxs, S, z);
+    return cudaSuccess;
+  }
+  // split-chain sums of y (chain-major) into out[0, hlen + 3), as ess_from_sums takes them
+  void chain_sums(const double* y, double* out) {
+    split_chain_stats<<<n_split, 256, hlen * sizeof(double), st>>>(y, n, hlen, split, mean, var, acov);
+    reduce_chains<<<(hlen + 1 + 255) / 256, 256, 0, st>>>(acov, mean, var, n_split, hlen, out);
+  }
+  void ess_rhat(const double* o, double* ess, double* rhat) const {
+    ess_from_sums(o, hlen, n_split, hlen, o[hlen], o[hlen + 1], o[hlen + 2], ess, rhat);
+  }
+};
 
 }  // namespace
 
@@ -276,71 +522,105 @@ int wn_ess_rhat(wn_handle* h, const double* draws, int64_t n_iter, int64_t n_cha
   const size_t per_rank = (size_t)n_iter * n_chains * dg;
   const size_t S = (size_t)W * n_iter * n_chains;
   if (S > 0x7ffffff0ull) return fail(h, WN_EUNSUPPORTED, "wn_ess_rhat: more than 2^31 draws per coordinate");
-  const int n_split = (int)((size_t)W * n_chains * (split ? 2 : 1));
   CUDA_TRY(h, cudaSetDevice(h->cfg.device));
   cudaStream_t st = h->stream;
-  double *d_in = nullptr, *d_all = nullptr, *d_x = nullptr, *d_xs = nullptr, *d_z = nullptr, *d_mean = nullptr,
-         *d_var = nullptr, *d_acov = nullptr, *d_out = nullptr;
-  unsigned *d_idx = nullptr, *d_idxs = nullptr;
-  void* d_tmp = nullptr;
-  size_t tmp_bytes = 0;
+  DevBufs bufs;
+  const double* src = nullptr;
+  int rc = pooled_draws(h, draws, per_rank, on_device, bufs, &src);
+  if (rc) return rc;
+  ColumnWork cw(W, n, (int)n_chains, dg, split, st);
+  double* d_out = nullptr;
+  ST_TRY(cw.alloc(bufs));
+  ST_TRY(bufs.alloc(&d_out, (size_t)hlen + 3));
   std::vector<double> out((size_t)hlen + 3);
-  int rc = WN_OK;
-  auto cleanup = [&]() {
-    cudaFree(d_in); cudaFree(d_all); cudaFree(d_x); cudaFree(d_xs); cudaFree(d_z); cudaFree(d_mean); cudaFree(d_var);
-    cudaFree(d_acov); cudaFree(d_out); cudaFree(d_idx); cudaFree(d_idxs); cudaFree(d_tmp);
-  };
-#define ST_TRY(expr)                                                                    \
-  do {                                                                                  \
-    cudaError_t _e = (expr);                                                            \
-    if (_e != cudaSuccess) {                                                            \
-      cleanup();                                                                        \
-      return fail(h, WN_ECUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));     \
-    }                                                                                   \
-  } while (0)
-  const double* src = draws;
-  if (!on_device) {
-    ST_TRY(cudaMalloc(&d_in, per_rank * sizeof(double)));
-    ST_TRY(cudaMemcpyAsync(d_in, draws, per_rank * sizeof(double), cudaMemcpyHostToDevice, st));
-    src = d_in;
-  }
-  if (W > 1) {
-    // the one collective of a multi-GPU run: every rank receives the monitored draws of all chains
-    ST_TRY(cudaMalloc(&d_all, per_rank * W * sizeof(double)));
-    ncclResult_t r = g_nccl.AllGather(src, d_all, per_rank, ncclDouble, (ncclComm_t)h->comm, st);
-    if (r != ncclSuccess) {
-      cleanup();
-      return fail(h, WN_ECUDA, std::string("ncclAllGather: ") + g_nccl.GetErrorString(r));
-    }
-    src = d_all;
-  }
-  ST_TRY(cudaMalloc(&d_x, S * sizeof(double)));
-  ST_TRY(cudaMalloc(&d_xs, S * sizeof(double)));
-  ST_TRY(cudaMalloc(&d_z, S * sizeof(double)));
-  ST_TRY(cudaMalloc(&d_idx, S * sizeof(unsigned)));
-  ST_TRY(cudaMalloc(&d_idxs, S * sizeof(unsigned)));
-  ST_TRY(cudaMalloc(&d_mean, (size_t)n_split * sizeof(double)));
-  ST_TRY(cudaMalloc(&d_var, (size_t)n_split * sizeof(double)));
-  ST_TRY(cudaMalloc(&d_acov, (size_t)n_split * hlen * sizeof(double)));
-  ST_TRY(cudaMalloc(&d_out, ((size_t)hlen + 3) * sizeof(double)));
-  ST_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, d_x, d_xs, d_idx, d_idxs, (int)S, 0, 64, st));
-  ST_TRY(cudaMalloc(&d_tmp, tmp_bytes));
-  ST_TRY(cudaFuncSetAttribute(split_chain_stats, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(hlen * sizeof(double))));
-  const int nb = (int)((S + 255) / 256 < 4096 ? (S + 255) / 256 : 4096);
-  for (int j = 0; j < dg && rc == WN_OK; ++j) {
-    gather_column<<<nb, 256, 0, st>>>(src, W, n, (int)n_chains, dg, j, d_x, d_idx);
-    ST_TRY(cub::DeviceRadixSort::SortPairs(d_tmp, tmp_bytes, d_x, d_xs, d_idx, d_idxs, (int)S, 0, 64, st));
-    rank_normalize<<<nb, 256, 0, st>>>(d_idxs, S, d_z);
-    split_chain_stats<<<n_split, 256, hlen * sizeof(double), st>>>(d_z, n, hlen, split ? 1 : 0, d_mean, d_var, d_acov);
-    reduce_chains<<<(hlen + 1 + 255) / 256, 256, 0, st>>>(d_acov, d_mean, d_var, n_split, hlen, d_out);
+  for (int j = 0; j < dg; ++j) {
+    cw.gather(src, j);
+    ST_TRY(cw.sort_rank(cw.x));
+    cw.chain_sums(cw.z, d_out);
     ST_TRY(cudaMemcpyAsync(out.data(), d_out, ((size_t)hlen + 3) * sizeof(double), cudaMemcpyDeviceToHost, st));
     ST_TRY(cudaStreamSynchronize(st));
-    ess_from_sums(out.data(), hlen, n_split, hlen, out[hlen], out[hlen + 1], out[hlen + 2], &ess[j], &rhat[j]);
+    cw.ess_rhat(out.data(), &ess[j], &rhat[j]);
   }
-#undef ST_TRY
-  cleanup();
-  return rc;
+  return WN_OK;
 }
+
+int wn_summary(wn_handle* h, const double* draws, int64_t n_iter, int64_t n_chains, int32_t dg, int on_device,
+               int32_t superchain_size, double* out) {
+  if (!h || !draws || !out || n_iter < 4 || n_chains < 1 || dg < 1 || superchain_size < 0)
+    return fail(h, WN_EINVAL, "wn_summary: need draws [n_iter >= 4, n_chains, dg], out [dg][WN_SUMMARY_COLS] and "
+                              "superchain_size >= 0");
+  const int W = h->comm ? h->comm_size : 1;
+  const int n = (int)n_iter;
+  const int hlen = n / 2;
+  if ((size_t)hlen * sizeof(double) > 200 * 1024) return fail(h, WN_EUNSUPPORTED, "wn_summary: more than 25 600 draws per split chain");
+  const size_t per_rank = (size_t)n_iter * n_chains * dg;
+  const size_t S = (size_t)W * n_iter * n_chains;
+  if (S > 0x7ffffff0ull) return fail(h, WN_EUNSUPPORTED, "wn_summary: more than 2^31 draws per coordinate");
+  const int M = W * (int)n_chains;   // chains over all ranks
+  const int s = superchain_size;
+  if (s > 0 && (M % s != 0 || M / s < 2))
+    return fail(h, WN_EINVAL, "wn_summary: the chains of all ranks must form at least 2 superchains of superchain_size");
+  CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+  cudaStream_t st = h->stream;
+  DevBufs bufs;
+  const double* src = nullptr;
+  int rc = pooled_draws(h, draws, per_rank, on_device, bufs, &src);
+  if (rc) return rc;
+  ColumnWork cw(W, n, (int)n_chains, dg, 1, st);
+  ST_TRY(cw.alloc(bufs));
+  // split-chain sums of six series: the ranks (bulk), x, 1[x <= q05], 1[x <= q95], (x - mean)^2 and the ranks of
+  // |x - q50|; then summary_moments' sc[6] and the nested R-hat
+  enum { BULK, RAW, I05, I95, SQ, FOLD, NSER };
+  const size_t L = (size_t)hlen + 3, n_out = NSER * L + 7;
+  double *d_out = nullptr, *d_y = nullptr, *d_part = nullptr;
+  unsigned* d_done = nullptr;
+  ST_TRY(bufs.alloc(&d_out, n_out));
+  ST_TRY(bufs.alloc(&d_y, S));
+  ST_TRY(bufs.alloc(&d_part, 4 * (size_t)cw.nb));
+  ST_TRY(bufs.alloc(&d_done, 1));
+  ST_TRY(cudaMemsetAsync(d_done, 0, sizeof(unsigned), st));
+  double* d_sc = d_out + NSER * L;
+  std::vector<double> o(n_out);
+  const double nan = std::nan("");
+  for (int j = 0; j < dg; ++j) {
+    cw.gather(src, j);
+    ST_TRY(cw.sort_rank(cw.x));
+    cw.chain_sums(cw.z, d_out + BULK * L);
+    summary_moments<<<cw.nb, 256, 0, st>>>(cw.xs, S, d_part, d_done, d_sc);
+    cw.chain_sums(cw.x, d_out + RAW * L);
+    for (int k = 0; k < 3; ++k) {
+      summary_series<<<cw.nb, 256, 0, st>>>(cw.x, S, d_sc, k, d_y);
+      cw.chain_sums(d_y, d_out + (I05 + k) * L);
+    }
+    summary_series<<<cw.nb, 256, 0, st>>>(cw.x, S, d_sc, 3, d_y);
+    ST_TRY(cw.sort_rank(d_y));   // overwrites the sorted column, which summary_moments has read
+    cw.chain_sums(cw.z, d_out + FOLD * L);
+    if (s > 0) {
+      chain_moments<<<(M + 7) / 8, 256, 0, st>>>(cw.x, n, M, cw.mean, cw.var);
+      nested_rhat<<<1, 256, 0, st>>>(cw.mean, cw.var, M / s, s, d_sc + 6);
+    }
+    ST_TRY(cudaMemcpyAsync(o.data(), d_out, n_out * sizeof(double), cudaMemcpyDeviceToHost, st));
+    ST_TRY(cudaStreamSynchronize(st));
+    double ess[NSER], rhat[NSER];
+    for (int k = 0; k < NSER; ++k) cw.ess_rhat(o.data() + k * L, &ess[k], &rhat[k]);
+    const double* sc = o.data() + NSER * L;
+    const double Sd = (double)S, sd = std::sqrt(sc[4] / (Sd - 1.0)), E = sc[4] / Sd;
+    double* r = out + (size_t)j * WN_SUMMARY_COLS;
+    r[WN_S_MEAN] = sc[0];
+    r[WN_S_SD] = sd;
+    r[WN_S_Q05] = sc[1];
+    r[WN_S_Q50] = sc[2];
+    r[WN_S_Q95] = sc[3];
+    r[WN_S_MCSE_MEAN] = sd / std::sqrt(ess[RAW]);
+    r[WN_S_MCSE_SD] = std::sqrt((sc[5] / Sd - E * E) / ess[SQ] / (4.0 * E));
+    r[WN_S_ESS_BULK] = ess[BULK];
+    r[WN_S_ESS_TAIL] = std::isnan(ess[I05]) || std::isnan(ess[I95]) ? nan : std::fmin(ess[I05], ess[I95]);
+    r[WN_S_RHAT] = std::isnan(rhat[BULK]) || std::isnan(rhat[FOLD]) ? nan : std::fmax(rhat[BULK], rhat[FOLD]);
+    r[WN_S_NESTED_RHAT] = s > 0 ? sc[6] : nan;
+  }
+  return WN_OK;
+}
+#undef ST_TRY
 
 int wn_moments_all(wn_handle* h, double* mean, double* var) {
   if (!h || !mean || !var) return fail(h, WN_EINVAL, "wn_moments_all: bad argument");

@@ -1,6 +1,7 @@
 """Cross-chain convergence diagnostics: bulk ESS and R-hat (Vehtari, Gelman, Simpson, Carpenter,
 Buerkner 2021), the quantities the reference's experiment scripts obtain from arviz
-(`az.ess`, WALNUTSpy_examples/gaussian/mainGaussESS.py:17,50-55).  arviz is not a dependency here.
+(`az.ess`, WALNUTSpy_examples/gaussian/mainGaussESS.py:17,50-55), and the posterior summary (`summary`: quantiles,
+MCSEs, tail ESS, folded R-hat, nested R-hat).  arviz is not a dependency here.
 
 Inputs are draws of ONE scalar quantity with shape (n_chains, n_draws), as numpy arrays or torch
 tensors (the same code runs on the GPU for the many-chain case: 65 536 chains x tens of draws).
@@ -112,6 +113,73 @@ def ess_bulk(x, split=True, max_lag=None):
         xp = _xp(z)
         z = xp.concatenate([z[:, :h], z[:, n - h:]], 0) if xp is np else xp.cat([z[:, :h], z[:, n - h:]], 0)
     return ess_from_stats(chain_stats(z, max_lag))
+
+
+def _split_ess(y):
+    """(ESS, R-hat) of y (n_chains, n) split into halves [0, h) and [n - h, n), h = n // 2, without rank
+    normalisation."""
+    n = y.shape[1]
+    h = n // 2
+    return ess_from_stats(chain_stats(np.concatenate([y[:, :h], y[:, n - h:]], 0)))
+
+
+def summary(x, superchain_size=None):
+    """Posterior summary of ONE quantity, draws x (n_chains, n_draws) with n_draws >= 4 (numpy; a torch tensor is
+    copied to the host): a dict of floats keyed mean, sd, q05, q50, q95, mcse_mean, mcse_sd, ess_bulk, ess_tail, rhat,
+    nested_rhat.  The host statement of what ChainBatch.summary / wn_summary compute on the device.
+
+    With M chains of N draws, S = M N, and "split ESS of y" = ESS of y with every chain split into [0, N // 2) and
+    [N - N // 2, N), without rank normalisation:
+      mean, sd       over all S draws, sd with 1 / (S - 1)
+      q05, q50, q95  np.quantile of the S draws (linear interpolation, numpy's default)
+      mcse_mean      sd / sqrt(split ESS of x)
+      mcse_sd        c = (x - mean)^2, E = mean(c), varvar = (mean(c^2) - E^2) / split ESS of c, sqrt(varvar / (4 E))
+      ess_bulk       ess_bulk(x)[0]: rank-normalised split ESS
+      ess_tail       min(split ESS of 1[x <= q05], split ESS of 1[x <= q95])
+      rhat           max(ess_bulk(x)[1], ess_bulk(|x - q50|)[1]): bulk and folded split-R-hat
+      nested_rhat    (superchain_size = s; chains k*s ... k*s + s - 1 form superchain k, K = M / s >= 2)
+                     sqrt(1 + B / W), B = 1/(K-1) sum_k (xbar_k - xbar)^2 over the superchain means,
+                     W = 1/K sum_k (Btilde_k + Wtilde_k), Btilde_k = 1/(s-1) sum_m (xbar_mk - xbar_k)^2 (0 if s = 1),
+                     Wtilde_k = 1/s sum_m var_mk (within-chain variance, 1 / (N - 1)); raw draws, not ranks.
+                     NaN without superchain_size (Margossian, Hoffman, Sountsov, Riou-Durand, Vehtari, Gelman 2024).
+    Ranks are ordinal and taken over all S draws before the split (for odd N the middle draw is ranked but dropped); an
+    ESS or R-hat of a series with zero variance is NaN, and so is every column computed from one (min / max are NaN
+    when either argument is).  ValueError for fewer than 4 draws or a superchain size that does not give at least 2
+    superchains."""
+    if _xp(x) is not np:
+        x = x.detach().cpu().numpy()
+    x = np.asarray(x, dtype=np.float64)
+    if x.ndim != 2 or x.shape[1] < 4:
+        raise ValueError("summary: draws must be (n_chains, n_draws >= 4)")
+    m, n = x.shape
+    s = int(superchain_size or 0)
+    if s < 0 or (s > 0 and (m % s != 0 or m // s < 2)):
+        raise ValueError(f"summary: {m} chains do not form at least 2 superchains of {superchain_size}")
+    S = x.size
+    with np.errstate(divide="ignore", invalid="ignore"):
+        mean = x.mean()
+        sd = np.sqrt(((x - mean) ** 2).sum() / (S - 1))
+        q05, q50, q95 = np.quantile(x.reshape(-1), [0.05, 0.5, 0.95])
+        ess_b, rhat_b = (np.float64(v) for v in ess_bulk(x))
+        rhat_f = np.float64(ess_bulk(np.abs(x - q50))[1])
+        ess_05 = np.float64(_split_ess((x <= q05).astype(np.float64))[0])
+        ess_95 = np.float64(_split_ess((x <= q95).astype(np.float64))[0])
+        c = (x - mean) ** 2
+        E = c.mean()
+        varvar = ((c * c).mean() - E * E) / np.float64(_split_ess(c)[0])
+        nested = np.float64("nan")
+        if s > 0:
+            xm = x.mean(1).reshape(-1, s)                      # chain means by superchain
+            xv = x.var(1, ddof=1).reshape(-1, s)
+            xk = xm.mean(1)
+            bt = ((xm - xk[:, None]) ** 2).sum(1) / (s - 1) if s > 1 else np.zeros_like(xk)
+            B = xk.var(ddof=1)
+            W = (bt + xv.mean(1)).mean()
+            nested = np.sqrt(1.0 + B / W)
+        return dict(mean=float(mean), sd=float(sd), q05=float(q05), q50=float(q50), q95=float(q95),
+                    mcse_mean=float(sd / np.sqrt(np.float64(_split_ess(x)[0]))), mcse_sd=float(np.sqrt(varvar / (4 * E))),
+                    ess_bulk=float(ess_b), ess_tail=float(np.minimum(ess_05, ess_95)),
+                    rhat=float(np.maximum(rhat_b, rhat_f)), nested_rhat=float(nested))
 
 
 def min_ess(draws, split=True, max_lag=None):

@@ -264,6 +264,21 @@ class ChainBatch:
         self._check(rc, "wn_ess_rhat")
         return ess, rhat
 
+    def summary(self, draws, superchain_size=None):
+        """Posterior summary of draws (n_iter, n_chains, dg) -- numpy or a torch CUDA tensor -- computed on the device:
+        a dict of [dg] arrays keyed mean, sd, q05, q50, q95, mcse_mean, mcse_sd, ess_bulk, ess_tail, rhat, nested_rhat
+        (definitions: include/walnuts_cuda.h at wn_summary; diagnostics.summary is the same on the host).  Pooled over
+        all ranks when a communicator is attached (one all-gather; global chain order is rank-major).
+        `superchain_size` = s: global chains k*s ... k*s + s - 1 form superchain k (start them from one point: repeat
+        each initial point s times in q0) and nested_rhat is computed; None leaves that column NaN.  ValueError if the
+        chains of all ranks do not form at least 2 superchains of s."""
+        n_iter, n_chains, dg = (int(x) for x in draws.shape)
+        p, dev = _ptr(draws, n_iter * n_chains * dg, what="summary(draws)")
+        out = np.empty((dg, len(_ffi.SUMMARY_COLS)))
+        rc = self._lib.wn_summary(self._h, p, n_iter, n_chains, dg, dev, int(superchain_size or 0), _ptr(out)[0])
+        self._check(rc, "wn_summary")
+        return {k: np.ascontiguousarray(out[:, i]) for i, k in enumerate(_ffi.SUMMARY_COLS)}
+
     def moments_all(self):
         """moments() over the chains of every rank of the communicator."""
         mean, var = np.empty(self.d), np.empty(self.d)
