@@ -64,6 +64,22 @@ def test_ess_rhat_of_sampler_draws(cuda_lib):
     assert (rhat < 1.01).all() and (ess > 0.3 * n * it).all()
 
 
+def test_moments_equal_moments_all_without_communicator(cuda_lib):
+    """Without a communicator wn_moments_all reduces over the handle's own chains: the same bits as wn_moments, and
+    numpy's mean and unbiased variance over the chains."""
+    from walnuts_b200 import ChainBatch
+    n, d = 1000, 37
+    rng = np.random.default_rng(21)
+    q = rng.standard_normal((n, d)) * np.logspace(-1, 1, d) + np.linspace(1.0, 20.0, d)
+    with ChainBatch("std_normal", d, n, H0=0.5, delta=0.3, M=5, seed=1) as cb:
+        cb.set_state(q)
+        mean, var = cb.moments()
+        mean_all, var_all = cb.moments_all()
+    assert np.array_equal(mean, mean_all) and np.array_equal(var, var_all)
+    assert np.all(np.abs(mean - q.mean(0)) <= 1e-12 * np.abs(q.mean(0)))
+    assert np.all(np.abs(var - q.var(0, ddof=1)) <= 1e-12 * q.var(0, ddof=1))
+
+
 def test_run_host_async_equals_run(cuda_lib):
     from walnuts_b200 import ChainBatch, pinned_empty
     n, d, it = 300, 9, 4

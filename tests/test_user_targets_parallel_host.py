@@ -20,6 +20,7 @@ WN_TARGET_LP_GRAD(q, g, data, n_data) {
   return 0.5 * lp;
 }"""
 FAM_PKG, FAM_EXT = 1, 3
+SMEM_MAX = 227 * 1024          # shared memory of one block on sm_100a
 
 # (d, G, E2, NT): the plan table at every boundary
 TABLE = [(1, 32, 4, 128), (256, 32, 4, 128), (257, 32, 8, 128), (512, 32, 8, 128), (513, 64, 8, 64),
@@ -52,7 +53,6 @@ def test_parallel_plan_table():
     with ThreadPoolExecutor(max_workers=min(len(TABLE), os.cpu_count() or 1)) as ex:
         tgs = list(ex.map(lambda r: targets.cuda_target(DIAG_SRC, r[0], name="plan_check", parallel=True), TABLE))
     for (d, G, E2, NT), tg in zip(TABLE, tgs):
-        assert targets.parallel_plan(d) == (G, E2, NT)
         totals = []
         for fam, is_pkg in ((FAM_EXT, 0), (FAM_PKG, 1)):
             shape, smem, pkg, total, dim = _plan(tg.plugin, fam)
@@ -60,8 +60,7 @@ def test_parallel_plan_table():
             # dynamic: checkpoint, reduction scratch, and per chain a q row, a g row (2 G E2 doubles each)
             assert smem == 8 * (3 * 2 * E2 * NT + 2 * ((G + 31) // 32) * 8 + (NT // G) * 2 * 2 * G * E2)
             totals.append(total)
-        # the host check computes exactly what the plug-in's static_assert computes
-        assert targets.parallel_smem_bytes(d, 0) == max(totals) <= targets.SMEM_MAX
+        assert max(totals) <= SMEM_MAX
 
 
 def test_parallel_refusals():
@@ -78,25 +77,21 @@ def test_parallel_refusals():
         targets.cuda_target(SEQ_SRC, 100, scratch=8)
 
 
-def _max_scratch(d):
-    from walnuts_b200 import targets
-    s = 0
-    while targets.parallel_smem_bytes(d, s + 1) <= targets.SMEM_MAX:
-        s += 1
-    return s
-
-
 def test_scratch_limit_agrees_with_the_plugin():
-    """The largest scratch the host check accepts compiles; one double more is refused by the host check AND by the
-    plug-in's static_assert (compiled directly, bypassing the host check)."""
+    """The largest scratch that fits by the plug-in's own accounting compiles; one double more is refused by
+    cuda_target (ValueError) and by the plug-in's static_assert (compiled directly)."""
     from walnuts_b200 import build, targets
     d = 4096
-    s = _max_scratch(d)
+    tg0 = targets.cuda_target(DIAG_SRC, d, name="plan_check", parallel=True)
+    (G, E2, NT), _, _, total_ext, _ = _plan(tg0.plugin, FAM_EXT)
+    total0 = max(total_ext, _plan(tg0.plugin, FAM_PKG)[3])
+    per_double = 8 * (NT // G)                  # one double of scratch per chain of the block
+    s = (SMEM_MAX - total0) // per_double
     assert s > 2000
     with pytest.raises(ValueError, match="scratch"):
         targets.cuda_target(DIAG_SRC, d, parallel=True, scratch=s + 1)
     tg = targets.cuda_target(DIAG_SRC, d, name="scratch_max", parallel=True, scratch=s)
-    assert _plan(tg.plugin, FAM_EXT)[3] == targets.parallel_smem_bytes(d, s) <= targets.SMEM_MAX
+    assert _plan(tg.plugin, FAM_EXT)[3] == total_ext + per_double * s <= SMEM_MAX
     csrc = os.path.join(build.HERE, "csrc")
     tu = (f"#define WN_USER_D {d}\n#define WN_USER_PARALLEL 1\n#define WN_USER_SCRATCH {s + 1}\n"
           f"#include \"wn_user_api.cuh\"\n{DIAG_SRC}\n#include \"wn_user_plugin.cuh\"\n")

@@ -69,22 +69,6 @@ static bool pick_plan(const wn_config& c, bool general, LaunchPlan& p, int& fam)
 // ------------------------------------------------------------------------------------------
 // small utility kernels
 // ------------------------------------------------------------------------------------------
-__global__ void moments_kernel(const double* __restrict__ state, int n_chains, int d,
-                               double* __restrict__ mean, double* __restrict__ var) {
-  const int j = blockIdx.x * blockDim.x + threadIdx.x;
-  if (j >= d) return;
-  double s = 0.0;
-  for (int c = 0; c < n_chains; ++c) s += state[(size_t)c * d + j];
-  const double m = s / n_chains;
-  double ss = 0.0;
-  for (int c = 0; c < n_chains; ++c) {
-    const double x = state[(size_t)c * d + j] - m;
-    ss = fma(x, x, ss);
-  }
-  mean[j] = m;
-  var[j] = n_chains > 1 ? ss / (n_chains - 1) : 0.0;
-}
-
 __global__ void transpose_kernel(const double* __restrict__ X, double* __restrict__ XT, int N, int P) {
   __shared__ double tile[32][33];
   const int n0 = blockIdx.x * 32, k0 = blockIdx.y * 32;
@@ -107,6 +91,188 @@ __global__ void fp64_fma_kernel(double* out, int iters, double a, double b) {
     x4 = fma(x4, a, b); x5 = fma(x5, a, b); x6 = fma(x6, a, b); x7 = fma(x7, a, b);
   }
   out[blockIdx.x * blockDim.x + threadIdx.x] = x0 + x1 + x2 + x3 + x4 + x5 + x6 + x7;
+}
+
+// ------------------------------------------------------------------------------------------
+// runs: check_run, then launch_geometry and launch
+// ------------------------------------------------------------------------------------------
+// Checks of a run request, made once by every wn_run* entry point before anything is staged or launched.
+// state_in: the call uploads the positions itself (wn_run_host_async with q_in).
+static int check_run(wn_handle* h, int64_t n_iter, bool state_in, const void* diag, const void* omin, const void* omax) {
+  if (!h) return WN_EINVAL;
+  const wn_config& c = h->cfg;
+  if ((omin == nullptr) != (omax == nullptr)) return fail(h, WN_EINVAL, "orbit_min and orbit_max go together");
+  if (omin && c.mode != WN_MODE_WALNUTSPY) return fail(h, WN_EINVAL, "orbit statistics exist in WALNUTSPY mode only");
+  if (diag && c.mode != WN_MODE_WALNUTSPY)
+    return fail(h, WN_EINVAL, "the 24-column diagnostics exist in WALNUTSPY mode only (walnuts.py returns draws only)");
+  if (n_iter <= 0 || n_iter > 0x7fffffff) return fail(h, WN_EINVAL, "n_iter must be positive");
+  if (!h->have_state && !state_in) return fail(h, WN_ESTATE, "wn_run before wn_set_state");
+  if (c.target == WN_TARGET_DIAG_GAUSS && !h->d_p0) return fail(h, WN_ESTATE, "diag_gauss needs data key inv_var");
+  if (c.target == WN_TARGET_LOGREG && (!h->d_p0 || !h->d_p1 || h->n_p1 != h->n_p0))
+    return fail(h, WN_ESTATE, "logreg needs data keys X [N*d] and y [N]");
+  if (c.target == WN_TARGET_STOCK_WATSON && (!h->d_p0 || h->n_p0 * 3 != c.d))
+    return fail(h, WN_ESTATE, "stock_watson needs data key y with T = d/3 entries");
+  if (c.target == WN_TARGET_DENSE_GAUSS && (!h->d_p0 || h->n_p0 != c.d))
+    return fail(h, WN_ESTATE, "dense_gauss needs data key precision [d*d]");
+  if (c.mode == WN_MODE_PACKAGE && !h->d_inv_mass) return fail(h, WN_ESTATE, "package mode needs data key inv_mass");
+  return WN_OK;
+}
+
+// Launch geometry of one run
+struct Geometry {
+  LaunchPlan p;
+  int fam;
+  int nslot;                     // resident chain slots (clusters for a cluster plan)
+  const UserTarget* ut;          // the plug-in that launches the kernel, or null
+  cudaLaunchConfig_t lc;         // grid, block, shared memory; the cluster attribute for a cluster plan only
+  cudaLaunchAttribute cluster;
+};
+
+// The plan of the run (general: see pick_plan), its grid and chain slots from the occupancy, and scratch for every slot
+// (grown, never shrunk)
+static int launch_geometry(wn_handle* h, bool general, Geometry& g) {
+  const wn_config& c = h->cfg;
+  if (!pick_plan(c, general, g.p, g.fam)) return fail(h, WN_EUNSUPPORTED, "no CUDA kernel for this target/dimension");
+  CUDA_TRY(h, cudaSetDevice(c.device));
+  g.ut = user_target(c.target);
+  int occ = 0;
+  if (g.ut) {
+    occ = g.ut->occupancy(user_family(c), c.device);
+    if (occ < 0) return fail(h, WN_ECUDA, "user target plug-in: occupancy query failed");
+  } else {
+    CUDA_TRY(h, cudaFuncSetAttribute(g.p.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.p.smem));
+    CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, g.p.fn, g.p.NT, g.p.smem));
+  }
+  if (occ < 1) return fail(h, WN_ECUDA, "kernel does not fit on an SM");
+  // G > NT: one chain per cluster of CL = G / NT blocks (wn_walnutspy.cuh); a slot is a cluster, and the resident
+  // cluster count comes from the runtime (how many clusters of CL blocks the GPCs hold), not from SMs x blocks per SM
+  const int cl = (g.p.G > g.p.NT) ? g.p.G / g.p.NT : 1;
+  g.cluster.id = cudaLaunchAttributeClusterDimension;
+  g.cluster.val.clusterDim.x = (unsigned)cl;
+  g.cluster.val.clusterDim.y = 1;
+  g.cluster.val.clusterDim.z = 1;
+  g.lc = {};
+  g.lc.blockDim = dim3(g.p.NT);
+  g.lc.dynamicSmemBytes = g.p.smem;
+  g.lc.stream = h->stream;
+  g.lc.attrs = &g.cluster;
+  g.lc.numAttrs = cl > 1;
+  long long blocks;
+  if (cl > 1) {
+    g.lc.gridDim = dim3((unsigned)cl);
+    int ncl = 0;
+    CUDA_TRY(h, cudaOccupancyMaxActiveClusters(&ncl, g.p.fn, &g.lc));
+    if (ncl < 1) return fail(h, WN_ECUDA, "no cluster of this kernel fits on the GPU");
+    const long long clusters = (ncl < c.n_chains) ? ncl : c.n_chains;
+    blocks = clusters * cl;
+    g.nslot = (int)clusters;
+  } else {
+    const int gpb = g.p.NT / g.p.G;
+    blocks = (long long)h->num_sms * occ;
+    const long long need = ((long long)c.n_chains + gpb - 1) / gpb;
+    if (blocks > need) blocks = need;
+    g.nslot = (int)blocks * gpb;
+  }
+  g.lc.gridDim = dim3((unsigned)blocks);
+  const int nvec = g.p.package ? package_scratch_vectors(c.M) : scratch_vectors(c.M);
+  const size_t sbytes = (size_t)nvec * g.p.E2 * g.nslot * g.p.G * sizeof(double2);
+  if (sbytes > h->scratch_bytes) {
+    if (h->d_scratch) cudaFree(h->d_scratch);
+    h->d_scratch = nullptr;
+    h->scratch_bytes = 0;
+    CUDA_TRY(h, cudaMalloc(&h->d_scratch, sbytes));
+    h->scratch_bytes = sbytes;
+  }
+  return WN_OK;
+}
+
+// The kernel launch of a run; params: the RunParams or PkgParams the plan's kernel takes.  A plug-in launches its own
+// kernels, which are registered in its statically linked CUDA runtime.
+static int launch(wn_handle* h, const Geometry& g, void* params) {
+  if (g.ut) {
+    const int rc = g.ut->launch(user_family(h->cfg), h->cfg.device, params, g.lc.gridDim.x, h->stream);
+    if (rc) return fail(h, WN_ECUDA, "user target plug-in: kernel launch failed (" + std::to_string(rc) + ")");
+    return WN_OK;
+  }
+  void* args[] = {params};
+  CUDA_TRY(h, cudaLaunchKernelExC(&g.lc, g.p.fn, args));
+  return WN_OK;
+}
+
+// the fields of RunParams and PkgParams that have the same name and meaning
+template <class Params>
+static void fill_queue_fields(Params& P, const wn_handle* h, int64_t n_iter, double* draws, int nslot,
+                              const unsigned int* order) {
+  const wn_config& c = h->cfg;
+  P.n_chains = c.n_chains; P.d = c.d; P.dg = c.dg; P.compat = c.compat;
+  P.n_iter = (int)n_iter; P.iter0 = h->iter_done + 1;
+  P.seed_lo = (uint32_t)(c.seed & 0xffffffffu); P.seed_hi = (uint32_t)(c.seed >> 32);
+  P.chain_offset = (uint32_t)c.chain_offset;
+  P.state = h->d_state; P.draws = draws; P.totals = h->d_totals;
+  P.scratch = h->d_scratch; P.nslot = nslot; P.queue = h->d_queue;
+  P.order = order; P.order_len = order ? h->d_sched_meta + 1 : nullptr; P.cost = h->d_cost;
+  P.tp.p0 = h->d_p0; P.tp.p1 = h->d_p1; P.tp.p2 = h->d_p2; P.tp.n0 = (int)h->n_p0; P.tp.n1 = (int)h->n_p1;
+  P.tp.c0 = (c.target == WN_TARGET_DIAG_GAUSS) ? h->inv_var_max : 1.0 / (h->tau * h->tau);
+  P.tp.c1 = (c.target == WN_TARGET_DIAG_GAUSS) ? h->inv_var_min : 0.0;
+}
+
+// a run that passed check_run, on device buffers
+static int run_async_impl(wn_handle* h, int64_t n_iter, double* d_draws, double* d_diag, uint64_t* d_nevalF,
+                          uint64_t* d_nevalB, double* d_omin, double* d_omax) {
+  const wn_config& c = h->cfg;
+  const bool adapting = h->d_adapt_state != nullptr && h->iter_done < (uint32_t)h->warmup_iter;
+  Geometry g;
+  if (const int rc = launch_geometry(h, adapting || d_omin != nullptr, g)) return rc;
+  CUDA_TRY(h, cudaMemsetAsync(h->d_queue, 0, sizeof(unsigned int), h->stream));
+  CUDA_TRY(h, cudaMemsetAsync(h->d_totals, 0, 2 * sizeof(unsigned long long), h->stream));
+
+  if (h->d_adapt_state && !adapting && !h->adapt_exported) {
+    // warm-up is over: freeze the adapted (H, delta) of every chain as its step size / tolerance
+    if (!h->d_H) CUDA_TRY(h, cudaMalloc(&h->d_H, (size_t)c.n_chains * sizeof(double)));
+    if (!h->d_delta) CUDA_TRY(h, cudaMalloc(&h->d_delta, (size_t)c.n_chains * sizeof(double)));
+    CUDA_TRY(h, cudaMemcpy2DAsync(h->d_H, sizeof(double), h->d_adapt_state, WN_ADAPT_STRIDE * sizeof(double),
+                                  sizeof(double), c.n_chains, cudaMemcpyDeviceToDevice, h->stream));
+    CUDA_TRY(h, cudaMemcpy2DAsync(h->d_delta, sizeof(double), h->d_adapt_state + 1, WN_ADAPT_STRIDE * sizeof(double),
+                                  sizeof(double), c.n_chains, cudaMemcpyDeviceToDevice, h->stream));
+    h->adapt_exported = true;
+  }
+  CUDA_TRY(h, cudaEventRecord(h->ev0, h->stream));
+  // queue order of this call: the chains that were longest in the previous call first (wn_sched.cu)
+  // -- for kernels whose chains share a warp (small d): there the per-chain cost is heavy-tailed and the gain measured
+  // (+3-4 % at config 3); with whole warps per chain it measured neutral (C2) to slightly negative (C4), so those keep
+  // the natural order
+  const unsigned int* order = nullptr;
+  if (g.p.G < 32)
+    if (const int src = wn_sched_prepare(h, g.nslot, 32 / g.p.G, &order)) return src;
+  RunParams P;
+  PkgParams K;
+  memset(&P, 0, sizeof(P)); memset(&K, 0, sizeof(K));
+  if (!g.p.package) {
+    fill_queue_fields(P, h, n_iter, d_draws, g.nslot, order);
+    P.M = c.M; P.kind = c.integrator; P.minC = c.minC; P.maxC = c.maxC;
+    P.H0 = c.H0; P.delta0 = c.delta; P.jitter = c.jitter; P.p0 = c.r2p_prob0;
+    P.log_p0 = c.log_p0; P.log_1mp0 = c.log_1mp0;
+    P.warmup_iter = h->warmup_iter; P.adaptH = h->adaptH; P.adaptDelta = h->adaptDelta;
+    P.p2prob = 1.0 - h->adHtarget; P.adTarget = h->adTarget; P.adQuant = h->adQuant;
+    P.adapt_state = h->d_adapt_state; P.adapt_hist = h->d_adapt_hist;
+    P.maxFPiter = h->maxFPiter; P.FPtol = h->FPtol; P.gradThresh = h->gradThresh;
+    // once adaptation has run, the adapted per-chain H / delta are the step sizes (WALNUTS.py:137,144)
+    P.Hstep = h->d_H; P.delta = h->d_delta; P.diag = d_diag;
+    P.orbit_min = d_omin; P.orbit_max = d_omax;
+    P.nevalF = (unsigned long long*)d_nevalF; P.nevalB = (unsigned long long*)d_nevalB;
+  } else {
+    fill_queue_fields(K, h, n_iter, d_draws, g.nslot, order);
+    K.max_depth = c.M; K.macro_step = c.H0; K.max_error = c.delta; K.inv_mass = h->d_inv_mass;
+    K.neval = (unsigned long long*)d_nevalF;
+  }
+  if (const int rc = launch(h, g, g.p.package ? (void*)&K : (void*)&P)) return rc;
+  CUDA_TRY(h, cudaEventRecord(h->ev1, h->stream));
+  if (h->d_cost) h->have_cost = true;
+  h->iter_done += (uint32_t)n_iter;
+  h->last_launches = 1;
+  h->last_plan[0] = g.fam; h->last_plan[1] = g.p.G; h->last_plan[2] = g.p.E2; h->last_plan[3] = g.p.NT;
+  h->last_slots = g.nslot;
+  return WN_OK;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -353,168 +519,10 @@ int wn_get_state(wn_handle* h, double* q, int on_device) {
   return WN_OK;
 }
 
-static int run_async_impl(wn_handle* h, int64_t n_iter, double* d_draws, double* d_diag, uint64_t* d_nevalF,
-                          uint64_t* d_nevalB, double* d_omin, double* d_omax);
-
 int wn_run_async(wn_handle* h, int64_t n_iter, double* d_draws, double* d_diag, uint64_t* d_nevalF,
                  uint64_t* d_nevalB) {
+  if (const int rc = check_run(h, n_iter, false, d_diag, nullptr, nullptr)) return rc;
   return run_async_impl(h, n_iter, d_draws, d_diag, d_nevalF, d_nevalB, nullptr, nullptr);
-}
-
-static int run_async_impl(wn_handle* h, int64_t n_iter, double* d_draws, double* d_diag, uint64_t* d_nevalF,
-                          uint64_t* d_nevalB, double* d_omin, double* d_omax) {
-  if (!h) return WN_EINVAL;
-  if ((d_omin == nullptr) != (d_omax == nullptr)) return fail(h, WN_EINVAL, "orbit_min and orbit_max go together");
-  if (d_omin && h->cfg.mode != WN_MODE_WALNUTSPY) return fail(h, WN_EINVAL, "orbit statistics exist in WALNUTSPY mode only");
-  if (d_diag && h->cfg.mode != WN_MODE_WALNUTSPY)
-    return fail(h, WN_EINVAL, "the 24-column diagnostics exist in WALNUTSPY mode only (walnuts.py returns draws only)");
-  if (n_iter <= 0 || n_iter > 0x7fffffff) return fail(h, WN_EINVAL, "n_iter must be positive");
-  if (!h->have_state) return fail(h, WN_ESTATE, "wn_run before wn_set_state");
-  const wn_config& c = h->cfg;
-  if (c.target == WN_TARGET_DIAG_GAUSS && !h->d_p0) return fail(h, WN_ESTATE, "diag_gauss needs data key inv_var");
-  if (c.target == WN_TARGET_LOGREG && (!h->d_p0 || !h->d_p1 || h->n_p1 != h->n_p0))
-    return fail(h, WN_ESTATE, "logreg needs data keys X [N*d] and y [N]");
-  if (c.target == WN_TARGET_STOCK_WATSON && (!h->d_p0 || h->n_p0 * 3 != c.d))
-    return fail(h, WN_ESTATE, "stock_watson needs data key y with T = d/3 entries");
-  if (c.target == WN_TARGET_DENSE_GAUSS && (!h->d_p0 || h->n_p0 != c.d))
-    return fail(h, WN_ESTATE, "dense_gauss needs data key precision [d*d]");
-  if (c.mode == WN_MODE_PACKAGE && !h->d_inv_mass) return fail(h, WN_ESTATE, "package mode needs data key inv_mass");
-  LaunchPlan p;
-  int fam;
-  const bool adapting = h->d_adapt_state != nullptr && h->iter_done < (uint32_t)h->warmup_iter;
-  if (!pick_plan(c, adapting || d_omin != nullptr, p, fam)) return fail(h, WN_EUNSUPPORTED, "no CUDA kernel for this target/dimension");
-  CUDA_TRY(h, cudaSetDevice(c.device));
-  const UserTarget* ut = user_target(c.target);
-  int occ = 0;
-  if (ut) {
-    occ = ut->occupancy(user_family(c), c.device);
-    if (occ < 0) return fail(h, WN_ECUDA, "user target plug-in: occupancy query failed");
-  } else {
-    CUDA_TRY(h, cudaFuncSetAttribute(p.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
-    CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, p.fn, p.NT, p.smem));
-  }
-  if (occ < 1) return fail(h, WN_ECUDA, "kernel does not fit on an SM");
-  // G > NT: one chain per cluster of CL = G / NT blocks (wn_walnutspy.cuh); a slot is a cluster, and the resident
-  // cluster count comes from the runtime (how many clusters of CL blocks the GPCs hold), not from SMs x blocks per SM
-  const int cl = (p.G > p.NT) ? p.G / p.NT : 1;
-  cudaLaunchAttribute cattr[1];
-  cattr[0].id = cudaLaunchAttributeClusterDimension;
-  cattr[0].val.clusterDim.x = (unsigned)cl;
-  cattr[0].val.clusterDim.y = 1;
-  cattr[0].val.clusterDim.z = 1;
-  cudaLaunchConfig_t lcfg = {};
-  lcfg.blockDim = dim3(p.NT);
-  lcfg.dynamicSmemBytes = p.smem;
-  lcfg.stream = h->stream;
-  lcfg.attrs = cattr;
-  lcfg.numAttrs = 1;
-  long long blocks;
-  int nslot;
-  if (cl > 1) {
-    lcfg.gridDim = dim3((unsigned)cl);
-    int ncl = 0;
-    CUDA_TRY(h, cudaOccupancyMaxActiveClusters(&ncl, p.fn, &lcfg));
-    if (ncl < 1) return fail(h, WN_ECUDA, "no cluster of this kernel fits on the GPU");
-    const long long clusters = (ncl < c.n_chains) ? ncl : c.n_chains;
-    blocks = clusters * cl;
-    nslot = (int)clusters;
-  } else {
-    const int gpb = p.NT / p.G;
-    blocks = (long long)h->num_sms * occ;
-    const long long need = ((long long)c.n_chains + gpb - 1) / gpb;
-    if (blocks > need) blocks = need;
-    nslot = (int)blocks * gpb;
-  }
-  const int nvec = p.package ? package_scratch_vectors(c.M) : scratch_vectors(c.M);
-  const size_t sbytes = (size_t)nvec * p.E2 * nslot * p.G * sizeof(double2);
-  if (sbytes > h->scratch_bytes) {
-    if (h->d_scratch) cudaFree(h->d_scratch);
-    h->d_scratch = nullptr;
-    h->scratch_bytes = 0;
-    CUDA_TRY(h, cudaMalloc(&h->d_scratch, sbytes));
-    h->scratch_bytes = sbytes;
-  }
-  CUDA_TRY(h, cudaMemsetAsync(h->d_queue, 0, sizeof(unsigned int), h->stream));
-  CUDA_TRY(h, cudaMemsetAsync(h->d_totals, 0, 2 * sizeof(unsigned long long), h->stream));
-
-  TargetParams tp;
-  tp.p0 = h->d_p0; tp.p1 = h->d_p1; tp.p2 = h->d_p2; tp.n0 = (int)h->n_p0; tp.n1 = (int)h->n_p1;
-  tp.c0 = (c.target == WN_TARGET_DIAG_GAUSS) ? h->inv_var_max : 1.0 / (h->tau * h->tau);
-  tp.c1 = (c.target == WN_TARGET_DIAG_GAUSS) ? h->inv_var_min : 0.0;
-
-  if (h->d_adapt_state && !adapting && !h->adapt_exported) {
-    // warm-up is over: freeze the adapted (H, delta) of every chain as its step size / tolerance
-    if (!h->d_H) CUDA_TRY(h, cudaMalloc(&h->d_H, (size_t)c.n_chains * sizeof(double)));
-    if (!h->d_delta) CUDA_TRY(h, cudaMalloc(&h->d_delta, (size_t)c.n_chains * sizeof(double)));
-    CUDA_TRY(h, cudaMemcpy2DAsync(h->d_H, sizeof(double), h->d_adapt_state, WN_ADAPT_STRIDE * sizeof(double),
-                                  sizeof(double), c.n_chains, cudaMemcpyDeviceToDevice, h->stream));
-    CUDA_TRY(h, cudaMemcpy2DAsync(h->d_delta, sizeof(double), h->d_adapt_state + 1, WN_ADAPT_STRIDE * sizeof(double),
-                                  sizeof(double), c.n_chains, cudaMemcpyDeviceToDevice, h->stream));
-    h->adapt_exported = true;
-  }
-  CUDA_TRY(h, cudaEventRecord(h->ev0, h->stream));
-  // queue order of this call: the chains that were longest in the previous call first (wn_sched.cu)
-  // -- for kernels whose chains share a warp (small d): there the per-chain cost is heavy-tailed and the gain measured
-  // (+3-4 % at config 3); with whole warps per chain it measured neutral (C2) to slightly negative (C4), so those keep
-  // the natural order
-  const unsigned int* order = nullptr;
-  if (p.G < 32)
-    if (const int src = wn_sched_prepare(h, nslot, 32 / p.G, &order)) return src;
-  if (!p.package) {
-    RunParams P;
-    memset(&P, 0, sizeof(P));
-    P.n_chains = c.n_chains; P.d = c.d; P.dg = c.dg; P.M = c.M; P.kind = c.integrator;
-    P.minC = c.minC; P.maxC = c.maxC; P.n_iter = (int)n_iter; P.iter0 = h->iter_done + 1;
-    P.compat = c.compat;
-    P.seed_lo = (uint32_t)(c.seed & 0xffffffffu); P.seed_hi = (uint32_t)(c.seed >> 32);
-    P.chain_offset = (uint32_t)c.chain_offset;
-    P.H0 = c.H0; P.delta0 = c.delta; P.jitter = c.jitter; P.p0 = c.r2p_prob0;
-    P.log_p0 = c.log_p0; P.log_1mp0 = c.log_1mp0;
-    P.warmup_iter = h->warmup_iter; P.adaptH = h->adaptH; P.adaptDelta = h->adaptDelta;
-    P.p2prob = 1.0 - h->adHtarget; P.adTarget = h->adTarget; P.adQuant = h->adQuant;
-    P.adapt_state = h->d_adapt_state; P.adapt_hist = h->d_adapt_hist;
-    P.maxFPiter = h->maxFPiter; P.FPtol = h->FPtol; P.gradThresh = h->gradThresh;
-    // once adaptation has run, the adapted per-chain H / delta are the step sizes (WALNUTS.py:137,144)
-    P.Hstep = h->d_H; P.delta = h->d_delta; P.state = h->d_state; P.draws = d_draws; P.diag = d_diag;
-    P.orbit_min = d_omin; P.orbit_max = d_omax;
-    P.nevalF = (unsigned long long*)d_nevalF; P.nevalB = (unsigned long long*)d_nevalB;
-    P.totals = h->d_totals; P.scratch = h->d_scratch; P.nslot = nslot; P.queue = h->d_queue; P.order = order; P.order_len = order ? h->d_sched_meta + 1 : nullptr; P.cost = h->d_cost; P.tp = tp;
-    void* args[] = {&P};
-    if (ut) {
-      const int rc = ut->launch(user_family(c), c.device, &P, (unsigned)blocks, h->stream);
-      if (rc) return fail(h, WN_ECUDA, "user target plug-in: kernel launch failed (" + std::to_string(rc) + ")");
-    } else if (cl > 1) {
-      lcfg.gridDim = dim3((unsigned)blocks);
-      CUDA_TRY(h, cudaLaunchKernelExC(&lcfg, p.fn, args));
-    } else {
-      CUDA_TRY(h, cudaLaunchKernel(p.fn, dim3((unsigned)blocks), dim3(p.NT), args, p.smem, h->stream));
-    }
-  } else {
-    PkgParams P;
-    memset(&P, 0, sizeof(P));
-    P.n_chains = c.n_chains; P.d = c.d; P.dg = c.dg; P.max_depth = c.M; P.compat = c.compat;
-    P.n_iter = (int)n_iter; P.iter0 = h->iter_done + 1;
-    P.seed_lo = (uint32_t)(c.seed & 0xffffffffu); P.seed_hi = (uint32_t)(c.seed >> 32);
-    P.chain_offset = (uint32_t)c.chain_offset;
-    P.macro_step = c.H0; P.max_error = c.delta; P.inv_mass = h->d_inv_mass;
-    P.state = h->d_state; P.draws = d_draws;
-    P.neval = (unsigned long long*)d_nevalF; P.totals = h->d_totals;
-    P.scratch = h->d_scratch; P.nslot = nslot; P.queue = h->d_queue; P.order = order; P.order_len = order ? h->d_sched_meta + 1 : nullptr; P.cost = h->d_cost; P.tp = tp;
-    void* args[] = {&P};
-    if (ut) {
-      const int rc = ut->launch(user_family(c), c.device, &P, (unsigned)blocks, h->stream);
-      if (rc) return fail(h, WN_ECUDA, "user target plug-in: kernel launch failed (" + std::to_string(rc) + ")");
-    } else {
-      CUDA_TRY(h, cudaLaunchKernel(p.fn, dim3((unsigned)blocks), dim3(p.NT), args, p.smem, h->stream));
-    }
-  }
-  CUDA_TRY(h, cudaEventRecord(h->ev1, h->stream));
-  if (h->d_cost) h->have_cost = true;
-  h->iter_done += (uint32_t)n_iter;
-  h->last_launches = 1;
-  h->last_plan[0] = fam; h->last_plan[1] = p.G; h->last_plan[2] = p.E2; h->last_plan[3] = p.NT;
-  h->last_slots = nslot;
-  return WN_OK;
 }
 
 int wn_sync(wn_handle* h) {
@@ -540,11 +548,9 @@ static int stage(wn_handle* h, double** buf, size_t* cap, size_t n) {
   return WN_OK;
 }
 
+// a run that passed check_run, on host buffers
 static int host_async_impl(wn_handle* h, int64_t n_iter, const double* q_in, double* draws, double* diag,
                            uint64_t* nevalF, uint64_t* nevalB, double* orbit_min, double* orbit_max, double* q_out) {
-  if (!h) return WN_EINVAL;
-  if ((orbit_min == nullptr) != (orbit_max == nullptr)) return fail(h, WN_EINVAL, "orbit_min and orbit_max go together");
-  if (n_iter <= 0 || n_iter > 0x7fffffff) return fail(h, WN_EINVAL, "n_iter must be positive");
   const wn_config& c = h->cfg;
   CUDA_TRY(h, cudaSetDevice(c.device));
   const size_t nd = draws ? (size_t)n_iter * c.n_chains * c.dg : 0;
@@ -580,15 +586,16 @@ static int host_async_impl(wn_handle* h, int64_t n_iter, const double* q_in, dou
 
 int wn_run_host_async(wn_handle* h, int64_t n_iter, const double* q_in, double* draws, double* diag,
                       uint64_t* nevalF, uint64_t* nevalB, double* q_out) {
+  if (const int rc = check_run(h, n_iter, q_in != nullptr, diag, nullptr, nullptr)) return rc;
   return host_async_impl(h, n_iter, q_in, draws, diag, nevalF, nevalB, nullptr, nullptr, q_out);
 }
 
 int wn_run_stats(wn_handle* h, int64_t n_iter, double* draws, double* diag, uint64_t* nevalF, uint64_t* nevalB,
                  double* orbit_min, double* orbit_max, int on_device) {
-  if (!h) return WN_EINVAL;
-  if ((orbit_min == nullptr) != (orbit_max == nullptr)) return fail(h, WN_EINVAL, "orbit_min and orbit_max go together");
-  int rc = on_device ? run_async_impl(h, n_iter, draws, diag, nevalF, nevalB, orbit_min, orbit_max)
-                     : host_async_impl(h, n_iter, nullptr, draws, diag, nevalF, nevalB, orbit_min, orbit_max, nullptr);
+  int rc = check_run(h, n_iter, false, diag, orbit_min, orbit_max);
+  if (rc) return rc;
+  rc = on_device ? run_async_impl(h, n_iter, draws, diag, nevalF, nevalB, orbit_min, orbit_max)
+                 : host_async_impl(h, n_iter, nullptr, draws, diag, nevalF, nevalB, orbit_min, orbit_max, nullptr);
   if (rc) return rc;
   return wn_sync(h);
 }
@@ -624,22 +631,6 @@ int wn_last_grad_evals(wn_handle* h, uint64_t* forward, uint64_t* backward) {
   if (!h) return WN_EINVAL;
   if (forward) *forward = h->last_tot[0];
   if (backward) *backward = h->last_tot[1];
-  return WN_OK;
-}
-
-int wn_moments(wn_handle* h, double* mean, double* var) {
-  if (!h || !mean || !var) return fail(h, WN_EINVAL, "wn_moments: bad argument");
-  if (!h->have_state) return fail(h, WN_ESTATE, "no state set");
-  const wn_config& c = h->cfg;
-  CUDA_TRY(h, cudaSetDevice(c.device));
-  double* buf = nullptr;
-  CUDA_TRY(h, cudaMalloc(&buf, 2 * (size_t)c.d * sizeof(double)));
-  moments_kernel<<<(c.d + 127) / 128, 128, 0, h->stream>>>(h->d_state, c.n_chains, c.d, buf, buf + c.d);
-  cudaError_t e = cudaMemcpyAsync(mean, buf, c.d * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(var, buf + c.d, c.d * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-  cudaFree(buf);
-  if (e != cudaSuccess) return fail(h, WN_ECUDA, cudaGetErrorString(e));
   return WN_OK;
 }
 

@@ -46,7 +46,7 @@ static LaunchPlan plan_pkg() {
   LaunchPlan p;
   p.fn = (const void*)package_kernel<T, G, E2, NT>;
   p.G = G; p.E2 = E2; p.NT = NT;
-  p.smem = (size_t)(3 * 2 * E2 * NT + 2 * ((G + 31) / 32) * 8 + T<G, E2>::smem_doubles(NT)) * sizeof(double);
+  p.smem = (size_t)pkg_smem_doubles<T, G, E2, NT>() * sizeof(double);
   p.package = true;
   return p;
 }

@@ -55,6 +55,12 @@ struct PkgCtl {
 
 #define WN_NEG_LOG3 (-1.0986122886681098)
 
+// dynamic shared memory of package_kernel in doubles: checkpoint, reduction scratch, target
+template <template <int, int> class TargetTT, int G, int E2, int NT>
+__host__ __device__ constexpr int pkg_smem_doubles() {
+  return 3 * 2 * E2 * NT + 2 * ((G + 31) / 32) * 8 + TargetTT<G, E2>::smem_doubles(NT);
+}
+
 template <template <int, int> class TargetTT, int G, int E2, int NT, int MINB = 1>
 __global__ void __launch_bounds__(NT, MINB) package_kernel(const __grid_constant__ PkgParams P) {
   constexpr int E = 2 * E2;

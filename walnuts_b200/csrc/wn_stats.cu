@@ -1,6 +1,7 @@
 // Cross-chain convergence statistics on the device, across GPUs: bulk ESS and split-R-hat of the monitored draws
 // (Vehtari, Gelman, Simpson, Carpenter, Buerkner 2021 -- the estimator behind arviz.ess, which the reference's
-// experiment scripts use: WALNUTSpy_examples/gaussian/mainGaussESS.py:17,50-55) and cross-GPU moments.
+// experiment scripts use: WALNUTSpy_examples/gaussian/mainGaussESS.py:17,50-55) and the cross-chain
+// moments of the state (wn_moments, wn_moments_all).
 //
 // Multi-GPU: chains shard across GPUs with no exchange while sampling; the ONE collective is an NCCL all-gather of the
 // monitored draws (wn_ess_rhat) or an all-reduce of (n, sum, sum of squares) (wn_moments_all).  NCCL is bound at run
@@ -409,15 +410,34 @@ struct ColumnWork {
   int W, n, n_chains, dg, hlen, split, n_split, nb;
   size_t S;
   cudaStream_t st;
+  const double* src;   // the pooled draws [W][n][n_chains][dg]
   double *x, *xs, *z, *mean, *var, *acov;
   unsigned *idx, *idxs;
   char* tmp = nullptr;
   size_t tmp_bytes = 0;
+  DevBufs bufs;        // every device buffer of the call
 
-  ColumnWork(int W_, int n_, int n_chains_, int dg_, int split_, cudaStream_t st_)
-      : W(W_), n(n_), n_chains(n_chains_), dg(dg_), hlen(split_ ? n_ / 2 : n_), split(split_ ? 1 : 0),
-        n_split(W_ * n_chains_ * (split_ ? 2 : 1)), S((size_t)W_ * n_ * n_chains_), st(st_) {
-    nb = (int)((S + 255) / 256 < 4096 ? (S + 255) / 256 : 4096);
+  // Argument checks, limits, the pooled draws and the buffers of a wn_ess_rhat / wn_summary call (`what`, named in
+  // every error message).  outs_ok: the caller's own arguments are valid, `outs` describes them.  s > 0: the chains of
+  // all ranks must form at least 2 superchains of s.
+  int setup(wn_handle* h, const char* what, bool outs_ok, const char* outs, const double* draws, int64_t n_iter,
+            int64_t n_chains_, int32_t dg_, int on_device, int split_, int s) {
+    if (!h || !draws || !outs_ok || n_iter < 4 || n_chains_ < 1 || dg_ < 1)
+      return fail(h, WN_EINVAL, std::string(what) + ": need draws [n_iter >= 4, n_chains, dg]" + outs);
+    W = h->comm ? h->comm_size : 1; n = (int)n_iter; n_chains = (int)n_chains_; dg = dg_; st = h->stream;
+    split = split_ ? 1 : 0; hlen = split ? n / 2 : n; n_split = W * n_chains * (split ? 2 : 1);
+    S = (size_t)W * n_iter * n_chains_; nb = (int)((S + 255) / 256 < 4096 ? (S + 255) / 256 : 4096);
+    if ((size_t)hlen * sizeof(double) > 200 * 1024)
+      return fail(h, WN_EUNSUPPORTED, std::string(what) + ": more than 25 600 draws per (split) chain");
+    if (S > 0x7ffffff0ull) return fail(h, WN_EUNSUPPORTED, std::string(what) + ": more than 2^31 draws per coordinate");
+    const int M = W * n_chains;
+    if (s > 0 && (M % s != 0 || M / s < 2))
+      return fail(h, WN_EINVAL, std::string(what) + ": the chains of all ranks must form at least 2 superchains of "
+                                                    "superchain_size");
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    if (const int rc = pooled_draws(h, draws, (size_t)n_iter * n_chains_ * dg_, on_device, bufs, &src)) return rc;
+    ST_TRY(alloc(bufs));
+    return WN_OK;
   }
   cudaError_t alloc(DevBufs& b) {
     cudaError_t e;
@@ -430,7 +450,7 @@ struct ColumnWork {
     return cudaFuncSetAttribute(split_chain_stats, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(hlen * sizeof(double)));
   }
   // column j of the pooled draws -> x (chain-major), idx = identity
-  void gather(const double* src, int j) { gather_column<<<nb, 256, 0, st>>>(src, W, n, n_chains, dg, j, x, idx); }
+  void gather(int j) { gather_column<<<nb, 256, 0, st>>>(src, W, n, n_chains, dg, j, x, idx); }
   // keys (chain-major) sorted with idx into xs / idxs; z = the rank-normalised keys, chain-major.  idx stays identity.
   cudaError_t sort_rank(const double* keys) {
     const cudaError_t e = cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, xs, idx, idxs, (int)S, 0, 64, st);
@@ -513,32 +533,20 @@ int wn_comm_destroy(wn_handle* h) {
 
 int wn_ess_rhat(wn_handle* h, const double* draws, int64_t n_iter, int64_t n_chains, int32_t dg, int on_device,
                 int32_t split, double* ess, double* rhat) {
-  if (!h || !draws || !ess || !rhat || n_iter < 4 || n_chains < 1 || dg < 1)
-    return fail(h, WN_EINVAL, "wn_ess_rhat: need draws [n_iter >= 4, n_chains, dg] and ess / rhat [dg]");
-  const int W = h->comm ? h->comm_size : 1;
-  const int n = (int)n_iter;
-  const int hlen = split ? n / 2 : n;
-  if ((size_t)hlen * sizeof(double) > 200 * 1024) return fail(h, WN_EUNSUPPORTED, "wn_ess_rhat: more than 25 600 draws per (split) chain");
-  const size_t per_rank = (size_t)n_iter * n_chains * dg;
-  const size_t S = (size_t)W * n_iter * n_chains;
-  if (S > 0x7ffffff0ull) return fail(h, WN_EUNSUPPORTED, "wn_ess_rhat: more than 2^31 draws per coordinate");
-  CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-  cudaStream_t st = h->stream;
-  DevBufs bufs;
-  const double* src = nullptr;
-  int rc = pooled_draws(h, draws, per_rank, on_device, bufs, &src);
-  if (rc) return rc;
-  ColumnWork cw(W, n, (int)n_chains, dg, split, st);
+  ColumnWork cw;
+  if (const int rc = cw.setup(h, "wn_ess_rhat", ess && rhat, " and ess / rhat [dg]", draws, n_iter, n_chains, dg,
+                              on_device, split, 0))
+    return rc;
+  const size_t L = (size_t)cw.hlen + 3;
   double* d_out = nullptr;
-  ST_TRY(cw.alloc(bufs));
-  ST_TRY(bufs.alloc(&d_out, (size_t)hlen + 3));
-  std::vector<double> out((size_t)hlen + 3);
+  ST_TRY(cw.bufs.alloc(&d_out, L));
+  std::vector<double> out(L);
   for (int j = 0; j < dg; ++j) {
-    cw.gather(src, j);
+    cw.gather(j);
     ST_TRY(cw.sort_rank(cw.x));
     cw.chain_sums(cw.z, d_out);
-    ST_TRY(cudaMemcpyAsync(out.data(), d_out, ((size_t)hlen + 3) * sizeof(double), cudaMemcpyDeviceToHost, st));
-    ST_TRY(cudaStreamSynchronize(st));
+    ST_TRY(cudaMemcpyAsync(out.data(), d_out, L * sizeof(double), cudaMemcpyDeviceToHost, cw.st));
+    ST_TRY(cudaStreamSynchronize(cw.st));
     cw.ess_rhat(out.data(), &ess[j], &rhat[j]);
   }
   return WN_OK;
@@ -546,44 +554,30 @@ int wn_ess_rhat(wn_handle* h, const double* draws, int64_t n_iter, int64_t n_cha
 
 int wn_summary(wn_handle* h, const double* draws, int64_t n_iter, int64_t n_chains, int32_t dg, int on_device,
                int32_t superchain_size, double* out) {
-  if (!h || !draws || !out || n_iter < 4 || n_chains < 1 || dg < 1 || superchain_size < 0)
-    return fail(h, WN_EINVAL, "wn_summary: need draws [n_iter >= 4, n_chains, dg], out [dg][WN_SUMMARY_COLS] and "
-                              "superchain_size >= 0");
-  const int W = h->comm ? h->comm_size : 1;
-  const int n = (int)n_iter;
-  const int hlen = n / 2;
-  if ((size_t)hlen * sizeof(double) > 200 * 1024) return fail(h, WN_EUNSUPPORTED, "wn_summary: more than 25 600 draws per split chain");
-  const size_t per_rank = (size_t)n_iter * n_chains * dg;
-  const size_t S = (size_t)W * n_iter * n_chains;
-  if (S > 0x7ffffff0ull) return fail(h, WN_EUNSUPPORTED, "wn_summary: more than 2^31 draws per coordinate");
-  const int M = W * (int)n_chains;   // chains over all ranks
   const int s = superchain_size;
-  if (s > 0 && (M % s != 0 || M / s < 2))
-    return fail(h, WN_EINVAL, "wn_summary: the chains of all ranks must form at least 2 superchains of superchain_size");
-  CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-  cudaStream_t st = h->stream;
-  DevBufs bufs;
-  const double* src = nullptr;
-  int rc = pooled_draws(h, draws, per_rank, on_device, bufs, &src);
-  if (rc) return rc;
-  ColumnWork cw(W, n, (int)n_chains, dg, 1, st);
-  ST_TRY(cw.alloc(bufs));
+  ColumnWork cw;
+  if (const int rc = cw.setup(h, "wn_summary", out && s >= 0, ", out [dg][WN_SUMMARY_COLS] and superchain_size >= 0",
+                              draws, n_iter, n_chains, dg, on_device, 1, s))
+    return rc;
+  const int n = cw.n, hlen = cw.hlen, M = cw.W * cw.n_chains;   // M: chains over all ranks
+  const size_t S = cw.S;
+  cudaStream_t st = cw.st;
   // split-chain sums of six series: the ranks (bulk), x, 1[x <= q05], 1[x <= q95], (x - mean)^2 and the ranks of
   // |x - q50|; then summary_moments' sc[6] and the nested R-hat
   enum { BULK, RAW, I05, I95, SQ, FOLD, NSER };
   const size_t L = (size_t)hlen + 3, n_out = NSER * L + 7;
   double *d_out = nullptr, *d_y = nullptr, *d_part = nullptr;
   unsigned* d_done = nullptr;
-  ST_TRY(bufs.alloc(&d_out, n_out));
-  ST_TRY(bufs.alloc(&d_y, S));
-  ST_TRY(bufs.alloc(&d_part, 4 * (size_t)cw.nb));
-  ST_TRY(bufs.alloc(&d_done, 1));
+  ST_TRY(cw.bufs.alloc(&d_out, n_out));
+  ST_TRY(cw.bufs.alloc(&d_y, S));
+  ST_TRY(cw.bufs.alloc(&d_part, 4 * (size_t)cw.nb));
+  ST_TRY(cw.bufs.alloc(&d_done, 1));
   ST_TRY(cudaMemsetAsync(d_done, 0, sizeof(unsigned), st));
   double* d_sc = d_out + NSER * L;
   std::vector<double> o(n_out);
   const double nan = std::nan("");
   for (int j = 0; j < dg; ++j) {
-    cw.gather(src, j);
+    cw.gather(j);
     ST_TRY(cw.sort_rank(cw.x));
     cw.chain_sums(cw.z, d_out + BULK * L);
     summary_moments<<<cw.nb, 256, 0, st>>>(cw.xs, S, d_part, d_done, d_sc);
@@ -622,8 +616,10 @@ int wn_summary(wn_handle* h, const double* draws, int64_t n_iter, int64_t n_chai
 }
 #undef ST_TRY
 
-int wn_moments_all(wn_handle* h, double* mean, double* var) {
-  if (!h || !mean || !var) return fail(h, WN_EINVAL, "wn_moments_all: bad argument");
+// Cross-chain mean and variance (1 / (n - 1)) of the current state; all_ranks: over the chains of every rank of the
+// communicator (without one, the handle's own chains)
+static int moments(wn_handle* h, double* mean, double* var, bool all_ranks, const char* what) {
+  if (!h || !mean || !var) return fail(h, WN_EINVAL, std::string(what) + ": bad argument");
   if (!h->have_state) return fail(h, WN_ESTATE, "no state set");
   const wn_config& c = h->cfg;
   CUDA_TRY(h, cudaSetDevice(c.device));
@@ -635,14 +631,14 @@ int wn_moments_all(wn_handle* h, double* mean, double* var) {
     cudaFree(buf);
     return fail(h, WN_ECUDA, msg);
   };
-  // two passes (sum -> mean, then centred sum of squares), each followed by ONE all-reduce when a communicator is set
+  // two passes (sum -> mean, then centred sum of squares), each followed by ONE all-reduce over the ranks
   for (int pass = 0; pass < 2; ++pass) {
     moment_sums<<<(d + 127) / 128, 128, 0, h->stream>>>(h->d_state, c.n_chains, d, pass ? buf + d + 1 : nullptr, buf);
     const double nloc = (double)c.n_chains;
     cudaError_t e = cudaMemcpyAsync(buf + d, &nloc, sizeof(double), cudaMemcpyHostToDevice, h->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);      // nloc is a stack variable
     if (e != cudaSuccess) return bail(cudaGetErrorString(e));
-    if (h->comm) {
+    if (all_ranks && h->comm) {
       ncclResult_t r = g_nccl.AllReduce(buf, buf, (size_t)d + 1, ncclDouble, ncclSum, (ncclComm_t)h->comm, h->stream);
       if (r != ncclSuccess) return bail(std::string("ncclAllReduce: ") + g_nccl.GetErrorString(r));
     }
@@ -662,5 +658,8 @@ int wn_moments_all(wn_handle* h, double* mean, double* var) {
   cudaFree(buf);
   return WN_OK;
 }
+
+int wn_moments(wn_handle* h, double* mean, double* var) { return moments(h, mean, var, false, "wn_moments"); }
+int wn_moments_all(wn_handle* h, double* mean, double* var) { return moments(h, mean, var, true, "wn_moments_all"); }
 
 }  // extern "C"

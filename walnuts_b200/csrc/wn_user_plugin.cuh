@@ -162,7 +162,8 @@ static_assert(WN_USER_PG <= WN_USER_PNT, "no thread-block clusters for user targ
 
 // Shared memory of the user kernels in bytes: the dynamic part of the plan plus the kernels' static __shared__
 // arrays (walnutspy_kernel: sh_bcast, sh_ctl, sh_ktab; package_kernel: sh_bcast, sh_ctl), each rounded up to 16 bytes.
-// walnuts_b200.targets.cuda_target() checks the same sum before it compiles anything.
+// The static_assert below is the one check of WN_USER_SCRATCH against the 227 KB of a block;
+// walnuts_b200.targets.cuda_target() reports its failure as a ValueError.
 constexpr size_t WN_SMEM_MAX = 227 * 1024;
 __host__ __device__ constexpr size_t round16(size_t b) { return (b + 15) / 16 * 16; }
 __host__ __device__ constexpr size_t user_static_smem(bool package, int G, int NT) {
@@ -176,8 +177,7 @@ constexpr size_t WN_USER_SMEM_EXT =
     (size_t)wpy_smem_doubles<UserParT, WN_USER_PG, WN_USER_PE2, WN_USER_PNT, true, KSET_ANY>() * sizeof(double) +
     user_static_smem(false, WN_USER_PG, WN_USER_PNT);
 constexpr size_t WN_USER_SMEM_PKG =
-    (size_t)(3 * 2 * WN_USER_PE2 * WN_USER_PNT + 2 * ((WN_USER_PG + 31) / 32) * 8 +
-             UserParT<WN_USER_PG, WN_USER_PE2>::smem_doubles(WN_USER_PNT)) * sizeof(double) +
+    (size_t)pkg_smem_doubles<UserParT, WN_USER_PG, WN_USER_PE2, WN_USER_PNT>() * sizeof(double) +
     user_static_smem(true, WN_USER_PG, WN_USER_PNT);
 static_assert(WN_USER_SMEM_EXT <= WN_SMEM_MAX && WN_USER_SMEM_PKG <= WN_SMEM_MAX,
               "cuda_target: WN_USER_SCRATCH too large, the plan's shared memory exceeds 227 KB per block");
@@ -217,7 +217,7 @@ int wn_user_plan(int family, int* G, int* E2, int* NT, size_t* smem, int* packag
 }
 
 // shared memory of the family's kernel per block in bytes: the plan's dynamic part plus the kernel's static arrays
-// (what cuda_target() checks against the 227 KB of a block before it compiles)
+// (the sum the static_assert above holds to the 227 KB of a block), for tests
 size_t wn_user_smem_total(int family) {
   const wn::LaunchPlan p = wn::user_plan(family);
   return p.smem + wn::user_static_smem(p.package, p.G, p.NT);

@@ -77,32 +77,6 @@ def logreg(X, y, tau=1.0):
     return Target("logreg", data={"X": X, "y": y, "tau": np.array([float(tau)])}, d=X.shape[1], ref="SURVEY.md T4")
 
 
-# Parallel protocol plans (wn_user_plugin.cuh, UserParT): (largest d, threads per chain G, coordinate pairs per thread
-# E2, threads per block NT) -- the shapes the built-in targets run on (wn_dispatch.cuh: pick_generic)
-PARALLEL_PLANS = [(256, 32, 4, 128), (512, 32, 8, 128), (1024, 64, 8, 64), (2048, 256, 4, 256), (4096, 512, 4, 512)]
-SMEM_MAX = 227 * 1024          # shared memory of one block on sm_100a
-_CTL_BYTES = 504               # sizeof(wn::Ctl), the per-warp control block of walnutspy_kernel
-
-
-def parallel_plan(d):
-    """(G, E2, NT) of a parallel-protocol user target of dimension d."""
-    for dmax, G, E2, NT in PARALLEL_PLANS:
-        if d <= dmax:
-            return G, E2, NT
-    raise ValueError(f"cuda_target(parallel=True): 1 <= d <= {PARALLEL_PLANS[-1][0]}")
-
-
-def parallel_smem_bytes(d, scratch):
-    """Shared memory per block of a parallel user target's kernels in bytes: the larger of the WALNUTSpy (EXT) and
-    package kernels, dynamic part plus static arrays, computed as the plug-in's static_assert computes it."""
-    G, E2, NT = parallel_plan(d)
-    r16 = lambda b: (b + 15) // 16 * 16
-    w = NT // 32
-    dyn = 3 * 2 * E2 * NT + 2 * ((G + 31) // 32) * 8 + (NT // G) * (2 * 2 * G * E2 + scratch)
-    # the package kernel has the same dynamic part and a smaller static one (its control block is smaller, no table)
-    return 8 * dyn + r16(4) + r16(_CTL_BYTES * w) + r16(4 * 32 * w)
-
-
 def cuda_target(source, d, data=None, name="user", verbose=False, *, parallel=False, scratch=0):
     """A user-defined target: the role of the reference's arbitrary Python `lpFun` (WALNUTSpy/targetDistr.py:18) /
     `logp`, `grad` (walnuts/walnuts.py:296-297) callables and of walnuts_stan.py's compiled Stan model.
@@ -130,8 +104,9 @@ def cuda_target(source, d, data=None, name="user", verbose=False, *, parallel=Fa
 
     Every thread of the chain must call ctx.sum and ctx.sync the same number of times in the same order (a call in a
     branch that differs between threads is undefined behaviour); indices j >= d are never handed out.  `scratch` is
-    limited by the 227 KB of shared memory of a block (parallel_smem_bytes).  Defining the macro of the other protocol
-    fails to compile with a message naming the right one.
+    limited by the 227 KB of shared memory of a block, which also holds the chains' q and g rows and the kernels' own
+    arrays: the plug-in checks the sum when it compiles, and a scratch too large raises ValueError.  Defining the
+    macro of the other protocol fails to compile with a message naming the right one.
 
     It is compiled once with nvcc for sm_100a into walnuts_b200/_lib/user/<hash>.so (cached by content), linked
     against the same persistent kernels as the built-in targets, and serves WALNUTS(...) with every integrator and the
@@ -140,15 +115,11 @@ def cuda_target(source, d, data=None, name="user", verbose=False, *, parallel=Fa
     d = int(d)
     scratch = int(scratch)
     if parallel:
-        if not 1 <= d <= PARALLEL_PLANS[-1][0]:
-            raise ValueError(f"cuda_target(parallel=True): 1 <= d <= {PARALLEL_PLANS[-1][0]} (one chain per warp up to "
-                             "d = 512, per block of 64 / 256 / 512 threads up to d = 1024 / 2048 / 4096)")
+        if not 1 <= d <= 4096:
+            raise ValueError("cuda_target(parallel=True): 1 <= d <= 4096 (one chain per warp up to d = 512, per block "
+                             "of 64 / 256 / 512 threads up to d = 1024 / 2048 / 4096)")
         if scratch < 0:
             raise ValueError("cuda_target: scratch must be >= 0 doubles")
-        need = parallel_smem_bytes(d, scratch)
-        if need > SMEM_MAX:
-            raise ValueError(f"cuda_target: scratch={scratch} needs {need} bytes of shared memory per block at d = {d}, "
-                             f"more than the {SMEM_MAX} of a block")
     else:
         if scratch != 0:
             raise ValueError("cuda_target: scratch needs parallel=True")
@@ -181,6 +152,9 @@ def cuda_target(source, d, data=None, name="user", verbose=False, *, parallel=Fa
             print(r.stderr)
         if r.returncode != 0:
             os.remove(src)
+            if "WN_USER_SCRATCH too large" in r.stdout + r.stderr:   # the plug-in's static_assert, in the front end
+                raise ValueError(f"cuda_target: scratch={scratch} does not fit at d = {d}: the kernels' shared memory "
+                                 "would exceed the 227 KB of a block")
             raise RuntimeError("cuda_target: nvcc failed:\n" + r.stdout + r.stderr)
         os.replace(src, so[:-3] + ".cu")
         os.replace(tmp, so)
